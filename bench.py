@@ -79,7 +79,14 @@ def parse_args():
     ap.add_argument("--cpu-threads", type=int, default=0)
     ap.add_argument("--wire-channels", type=int, default=-1,
                     help="streams of the wire-level leg (unmodified server + its own grpc_load_test.py); 0 = skip, -1 = 64 at N = 1")
-    return resolve_config(ap.parse_args())
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step decoded (rank 0's windows) to DIR/<name>.npy, for comparing two builds")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return resolve_config(args)
 
 
 def resolve_config(args):
@@ -120,6 +127,23 @@ def window_lengths(rank: int, sessions: int, kind: str = "partial"):
         return [30.0] * sessions
     lo, hi = (2.0, 10.0) if kind == "partial" else (1.0, 8.0)  # utterance: the burst lengths of tools/stream_bench.py
     return [float(np.round(rng.uniform(lo, hi), 2)) for _ in range(sessions)]
+
+
+def dump_outputs(out_dir: str, results, lengths) -> None:
+    """The decoded result of every window as a caller of the decode path receives it (tokens cut at the first EOT,
+    padded with -1; sum / average log-probability), plus the window lengths it came from.  No no-speech probability:
+    the timed pipeline starts decoding after the prompt and never computes one."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = max([len(r["tokens"]) for r in results] + [1])
+    tokens = np.full((len(results), n), -1.0, dtype=np.float64)
+    for i, r in enumerate(results):
+        tokens[i, :len(r["tokens"])] = r["tokens"]
+    arrays = {"tokens": tokens, "n_tokens": np.array([len(r["tokens"]) for r in results], dtype=np.float64),
+              "sum_logprob": np.array([r["sum_logprob"] for r in results], dtype=np.float32),
+              "avg_logprob": np.array([r["avg_logprob"] for r in results], dtype=np.float32),
+              "window_seconds": np.array(lengths, dtype=np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def faster_whisper_row():
@@ -352,6 +376,8 @@ def run_b200(args):
     total_ms = barrier_max(dist, local, total_ms)
     clocks = sampler.stop() if sampler else None
     ms_per_step = total_ms / args.steps
+    if args.dump_outputs and rank == 0:  # before the e2e leg reuses the engine's decoder state
+        dump_outputs(args.dump_outputs, eng.bench_pipeline_results(S, NG, n_steps, args.profile["length_penalty"]), lengths)
 
     # ---- e2e: public backend call from S host threads, host buffers ----
     lat = []

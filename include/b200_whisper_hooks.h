@@ -33,6 +33,10 @@ int bw_bench_decoder_step(bw_engine*, int32_t n_segments, int32_t n_group, int32
  * CUDA-event pair on the engine stream; returns total ms. */
 int bw_bench_pipeline(bw_engine*, const float* pcm_host, const int64_t* offsets, const int64_t* lengths,
                       int32_t n_segments, int32_t n_group, int32_t n_steps, float* ms_out);
+/* What the last bw_bench_pipeline call (same n_segments, n_group, n_steps) decoded: one bw_result per window, finalised
+ * as bw_call_decode finalises a beam-search request (length_penalty < 0: none, as in bw_decode_opts). Untimed. */
+int bw_bench_pipeline_results(bw_engine*, int32_t n_segments, int32_t n_group, int32_t n_steps, float length_penalty,
+                              bw_result* out);
 
 /* Test hook for the decoder LayerNorm fusion (device pointers): producer row GEMM x = res + A.Wp^T + bp (also
  * emits bf16(x) and per-row LayerNorm partials) then consumer row GEMM out = [gelu](LayerNorm(x; gamma, beta).Wc^T + bc)

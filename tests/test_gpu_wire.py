@@ -3,8 +3,9 @@
 (stt_server/backend/application/model_registry.py:385-680) and the whole unmodified server over gRPC (CreateSession +
 StreamingRecognize) under its own load generator tools/bench/grpc_load_test.py -- drive `B200WhisperBackend` on cuda:0.
 
-The GPU box has no /root/reference: the reference is installed (unmodified) under the git-ignored baseline/_ref by
-tools/install_reference.sh and travels with the snapshot.  Skipped when neither is present."""
+The upstream server and its load generator are not part of this repository: these tests run where a checkout is found
+($STT_SERVER_ROOT, or the unmodified install tools/install_reference.sh makes under the git-ignored baseline/_ref) and
+skip elsewhere."""
 import json
 import os
 import subprocess
@@ -24,7 +25,8 @@ from wire_bench import reference_layout  # noqa: E402
 
 LAYOUT = reference_layout()
 if LAYOUT is None:
-    pytest.skip("no reference tree: run tools/install_reference.sh", allow_module_level=True)
+    pytest.skip("needs the upstream server source (stt_server, tools/bench/grpc_load_test.py), which is not part of this "
+                "repository: set STT_SERVER_ROOT or run tools/install_reference.sh", allow_module_level=True)
 PKG_ROOT, TREE = LAYOUT
 
 from b200_whisper.backend import B200WhisperBackend  # noqa: E402

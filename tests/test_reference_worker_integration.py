@@ -1,7 +1,9 @@
 """The drop-in claim against the REAL caller: the reference's own `ModelWorker` (stt_server/model/worker.py) resolves
 `backend="b200_whisper"` through its registry, constructs `B200WhisperBackend` the way it constructs its own backends and
-drives it through `decode_sync` -- bytes in, `DecodeResult` out.  Runs wherever the reference tree is mounted (the build
-container); the GPU box has no /root/reference, so the engine below the backend is the host-logic fake (no CUDA here)."""
+drives it through `decode_sync` -- bytes in, `DecodeResult` out.  The upstream source is not part of this repository: the
+tests that import it run where a checkout is found ($STT_SERVER_ROOT, or the install tools/install_reference.sh makes) and
+skip elsewhere.  The engine below the backend is the host-logic fake (no CUDA needed).  The run-time proto stubs are
+checked on a stored wire schema (tests/golden/stt_wire.proto) everywhere, and on the upstream proto where it is found."""
 import os
 import sys
 import time
@@ -15,13 +17,20 @@ from b200_whisper.vocab import vocab_for
 from tests._util import ACCURATE, REALTIME
 from tests.test_host_logic import FakeEngine, res
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "stt_server")), reason="reference tree not mounted")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+from wire_bench import reference_layout  # noqa: E402
+
+LAYOUT = reference_layout()
+PKG_ROOT, TREE = LAYOUT or (None, None)  # upstream package root (for sys.path), directory holding its config/ and proto/
+needs_upstream = pytest.mark.skipif(LAYOUT is None, reason="needs the upstream server source (stt_server), which is not part of "
+                                                           "this repository: set STT_SERVER_ROOT or run tools/install_reference.sh")
+STORED_PROTO = os.path.join(ROOT, "tests", "golden", "stt_wire.proto")
 
 
 @pytest.fixture
 def reference_worker(monkeypatch):
-    monkeypatch.syspath_prepend(REF)
+    monkeypatch.syspath_prepend(PKG_ROOT)
     for name in [n for n in sys.modules if n == "stt_server" or n.startswith("stt_server.")]:
         monkeypatch.delitem(sys.modules, name)
     from b200_whisper import register
@@ -53,6 +62,7 @@ def _pcm(seed, seconds, rate=16000):
     return (np.clip(a, -1, 1) * 32767).astype(np.int16).tobytes()
 
 
+@needs_upstream
 def test_real_model_worker_drives_the_backend(reference_worker):
     worker, eng, audios = reference_worker
     assert worker.get_backend("b200_whisper") is bk.B200WhisperBackend
@@ -92,6 +102,7 @@ def test_real_model_worker_drives_the_backend(reference_worker):
     w.close()
 
 
+@needs_upstream
 def test_real_worker_pool_shares_one_engine(reference_worker, monkeypatch):
     """model_registry.py:230-247 builds pool_size workers with identical arguments: every handle must share one engine."""
     worker, eng, _ = reference_worker
@@ -106,10 +117,16 @@ def test_real_worker_pool_shares_one_engine(reference_worker, monkeypatch):
 
 
 def test_runtime_proto_stubs_roundtrip():
-    """protostubs.install builds stt_pb2 / stt_pb2_grpc from the reference's proto/stt.proto without grpc_tools."""
+    """protostubs builds stt_pb2 / stt_pb2_grpc from a .proto without grpc_tools: the stored wire schema, and the upstream
+    proto/stt.proto where a checkout is found."""
+    for path in [STORED_PROTO] + ([os.path.join(TREE, "proto", "stt.proto")] if TREE else []):
+        _check_proto_stubs(path)
+
+
+def _check_proto_stubs(path):
     from b200_whisper import protostubs
 
-    pb2 = protostubs.build_pb2_module(protostubs.parse_proto(open(os.path.join(REF, "proto", "stt.proto")).read()), "x_pb2")
+    pb2 = protostubs.build_pb2_module(protostubs.parse_proto(open(path).read()), "x_pb2")
     grpc_mod = protostubs.build_grpc_module(pb2, "x_pb2_grpc")
     req = pb2.SessionRequest(session_id="s", vad_mode=pb2.VAD_AUTO_END, task=pb2.TASK_TRANSLATE, decode_profile=pb2.DECODE_PROFILE_ACCURATE)
     req.attributes["k"] = "v"
@@ -127,6 +144,7 @@ def test_runtime_proto_stubs_roundtrip():
     assert all(hasattr(grpc_mod, n) for n in ("STTBackendStub", "STTBackendServicer", "add_STTBackendServicer_to_server"))
 
 
+@needs_upstream
 def test_real_model_registry_dispatches_to_the_backend(reference_worker, monkeypatch):
     """SURVEY 8a row a1 with the REAL code: `ModelRegistry.load_model` builds a pool of `b200_whisper` workers, and
     `submit_decode` / `_dispatch_loop` / `_worker_loop` (model_registry.py:385-680) call `transcribe` from pool_size threads at
@@ -136,7 +154,7 @@ def test_real_model_registry_dispatches_to_the_backend(reference_worker, monkeyp
     from b200_whisper import protostubs
 
     worker, eng, _ = reference_worker
-    protostubs.install(os.path.join(REF, "proto", "stt.proto"))
+    protostubs.install(os.path.join(TREE, "proto", "stt.proto"))
     from stt_server.backend.application.model_registry import ModelRegistry
 
     lock = threading.Lock()
@@ -192,6 +210,7 @@ def _free_port():
     return port
 
 
+@needs_upstream
 def test_unmodified_server_end_to_end_over_grpc(tmp_path):
     """The wire-level drop-in (SURVEY 8(f) row 4): the UNMODIFIED reference server -- gRPC servicer, session manager, stream
     orchestrator, decode scheduler, model registry, ModelWorker -- started by `b200_whisper.launcher` with
@@ -206,14 +225,14 @@ def test_unmodified_server_end_to_end_over_grpc(tmp_path):
     port, mport, wport = _free_port(), _free_port(), _free_port()
     cfg = tmp_path / "server.yaml"
     # the shipped server configuration (limits, partial-decode schedule, ...) + a loopback WebSocket port of our own
-    cfg.write_text(open(os.path.join(REF, "config", "server.yaml")).read() + f"\nws_host: 127.0.0.1\nws_port: {wport}\n")
+    cfg.write_text(open(os.path.join(TREE, "config", "server.yaml")).read() + f"\nws_host: 127.0.0.1\nws_port: {wport}\n")
     repo = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     proc = subprocess.Popen(
         [sys.executable, os.path.join(repo, "tests", "_ref_server_driver.py"), "--config", str(cfg), "--model-backend", "b200_whisper",
          "--model", "random:test-tiny", "--device", "cuda:0", "--port", str(port), "--metrics-port", str(mport),
          "--vad-threshold", "0", "--model-pool-size", "2", "--language", "en", "--log-level", "INFO"],
-        cwd=repo, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-    pb2 = protostubs.build_pb2_module(protostubs.parse_proto(open(os.path.join(REF, "proto", "stt.proto")).read()), "client_pb2")
+        cwd=repo, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, env=dict(os.environ, STT_SERVER_ROOT=PKG_ROOT))
+    pb2 = protostubs.build_pb2_module(protostubs.parse_proto(open(os.path.join(TREE, "proto", "stt.proto")).read()), "client_pb2")
     pb2_grpc = protostubs.build_grpc_module(pb2, "client_pb2_grpc")
     results, log = [], ""
     try:

@@ -97,6 +97,7 @@ SIGNATURES = {
     "bw_bench_mel": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, c_f32_p, C.POINTER(C.c_double)]),
     "bw_bench_pipeline": (C.c_int, [C.c_void_p, c_f32_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_int32, C.c_int32,
                                     C.c_int32, c_f32_p]),
+    "bw_bench_pipeline_results": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.POINTER(ResultC)]),
     "bw_bench_decoder_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, c_f32_p,
                                         C.POINTER(C.c_double)]),
     "bw_test_ln_chain": (C.c_int, [C.c_void_p] * 8 + [C.c_int32] * 5 + [C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -294,6 +294,41 @@ int bw_bench_pipeline(bw_engine* e, const float* pcm_host, const int64_t* offset
   BW_API_END
 }
 
+// What the last bw_bench_pipeline decoded (same n_segments / n_group / n_steps), finalised per window as a decode
+// request's result: the pipeline leaves window i's decoder state in request slot i, sequences i * n_group onwards.
+int bw_bench_pipeline_results(bw_engine* e, int32_t n_segments, int32_t n_group, int32_t n_steps, float length_penalty,
+                              bw_result* out) {
+  BW_API_BEGIN
+  BW_CHECK(e && out, "bad argument");
+  BW_CHECK(e->state == 1, "engine not finalized");
+  BW_CHECK(n_segments >= 1 && n_segments <= e->Q && n_group >= 1 && n_group <= kMaxBeam && n_segments * n_group <= e->S, "exceeds pools");
+  BW_CHECK(n_steps >= 1 && 3 + n_steps < e->dims.n_text_ctx, "n_steps out of range");
+  DeviceGuard dg(e->device);
+  std::lock_guard<std::mutex> g(e->gpu_mu);
+  BW_CHECK(e->live.empty(), "engine busy");
+  const size_t blob = fin_blob_bytes(e);
+  for (int i = 0; i < n_segments; ++i) {
+    int* rec = e->h_init + i * 3;
+    rec[0] = i; rec[1] = i * n_group; rec[2] = n_group;
+  }
+  BW_CUDA(cudaMemcpyAsync(e->d_init.p, e->h_init, (size_t)n_segments * 12, cudaMemcpyHostToDevice, e->stream));
+  engine_gather_final(e, e->d_init.as<int>(), n_segments, (int)blob, e->d_fin.as<unsigned char>());
+  BW_CUDA(cudaMemcpyAsync(e->h_fin, e->d_fin.p, (size_t)n_segments * blob, cudaMemcpyDeviceToHost, e->stream));
+  BW_CUDA(cudaStreamSynchronize(e->stream));
+  for (int i = 0; i < n_segments; ++i) {
+    Request r;  // as synthetic_init admitted it: 3 prompt tokens, beam-search bookkeeping, then n_steps steps
+    r.initial.assign(3, 0);
+    r.greedy = 0;
+    r.G = n_group;
+    r.cur_len = 3 + n_steps;
+    r.steps = n_steps;
+    r.length_penalty = length_penalty;
+    r.out = out + i;
+    finalize_decode(e, &r, e->h_fin + (size_t)i * blob);
+  }
+  BW_API_END
+}
+
 // The decoder step's dominant kernel alone: cross-attention of one layer over resident K/V.
 int bw_bench_cross_attention(bw_engine* e, int32_t n_segments, int32_t n_group, int32_t iters, float* ms_out, double* bytes_out) {
   BW_API_BEGIN

@@ -72,6 +72,8 @@ int submit_many_and_wait(bw_engine* e, const std::vector<Request*>& rs);
 // validates `opts` and fills the decode fields of `r` (shared by bw_call_decode, bw_decode_many and the test hooks)
 void fill_decode_request(Request& r, bw_call* c, int seek, const bw_decode_opts* o, bw_result* out);
 size_t fin_blob_bytes(bw_engine* e);
+// one finished request's blob (engine_gather_final) -> r->out: the ranker's pick among the request's hypotheses
+void finalize_decode(bw_engine* e, Request* r, const unsigned char* blob);
 
 }  // namespace bw
 

@@ -219,6 +219,8 @@ int find_seq_block(bw_engine* e, int G) {
   return -1;
 }
 
+}  // namespace
+
 // host-side finalisation: BeamSearchDecoder.finalize / GreedyDecoder.finalize + MaximumLikelihoodRanker
 void finalize_decode(bw_engine* e, Request* r, const unsigned char* blob) {
   const int n_ctx = e->dims.n_text_ctx;
@@ -293,8 +295,6 @@ void finalize_decode(bw_engine* e, Request* r, const unsigned char* blob) {
   o->no_speech_prob = fmisc[0];
   o->n_steps = r->steps;
 }
-
-}  // namespace
 
 size_t fin_blob_bytes(bw_engine* e) {
   return (size_t)kMaxFinished * 12 + 4 + 4 + kMaxBeam * 4 + (size_t)e->dims.n_text_ctx * kMaxBeam * 4 +

@@ -320,6 +320,14 @@ class Engine:
                                            n_steps, C.byref(ms)), "bw_bench_pipeline")
         return ms.value
 
+    def bench_pipeline_results(self, n_segments: int, n_group: int, n_steps: int, length_penalty: Optional[float]) -> list:
+        """Result dicts (as decode_many returns them) of every window of the last bench_pipeline call with these arguments."""
+        results = (L.ResultC * n_segments)()
+        L.check(self.lib.bw_bench_pipeline_results(self.handle, n_segments, n_group, n_steps,
+                                                   -1.0 if length_penalty is None else float(length_penalty), results),
+                "bw_bench_pipeline_results")
+        return [result_dict(r) for r in results]
+
     def retain(self) -> None:
         self.lib.bw_engine_retain(self.handle)
 
