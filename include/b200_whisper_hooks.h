@@ -19,6 +19,40 @@ extern "C" {
  * 2 = tcgen05 swap-AB (the decoder's skinny-GEMM path) */
 int bw_gemm_bf16(int impl, const void* A, const void* B, void* C, const float* bias, const float* residual,
                  int32_t M, int32_t N, int32_t K, int32_t gelu, int32_t out_fp32, void* stream);
+/* A GEMM in the argument form the engine launches (bw::GemmArgs): for z < Z,
+ *   D_z[i][j] = [gelu](sum_k A_z[i][k] * B_z[j][k] + bias_z[j]) (+ residual_z[i][j])      i < M, j < N
+ * with X_z = X + z * x_zstride (elements; a zero stride with Z > 1 broadcasts one slice), leading dimensions lda / ldb
+ * / ldc / ldres, and a_rows / b_rows (>= M / N; 0 = M / N) rows allocated behind A / B.  transposed stores D^T
+ * (C[j * ldc + i], bias_z[i], residual_z[j * ldres + i]).  Device pointers; bias and residual are fp32 or NULL. */
+typedef struct bw_gemm_desc {
+  const void* A;
+  const void* B;
+  void* C;
+  const float* bias;
+  const float* residual;
+  int32_t M, N, K;
+  int32_t lda, ldb, ldc, ldres;
+  int32_t Z;
+  int32_t a_rows, b_rows;
+  int64_t a_zstride, b_zstride, c_zstride, bias_zstride, res_zstride;
+  int32_t gelu, out_fp32, transposed;
+} bw_gemm_desc;
+/* GEMM kernel routes: BW_GEMM_ROUTE(kernel, param) with the K split of the split-K / row kernels (row KS 1 = the
+ * unsplit row kernel), the tile width of the plain tile kernel, 0 for the pair and SIMT kernels. */
+#define BW_GEMM_PAIR 1   /* persistent CTA-pair kernel (cta_group::2, 256x256 tiles) */
+#define BW_GEMM_SPLITK 2 /* cluster split-K kernel, DSMEM pull reduction; KS 2 / 4 / 8 */
+#define BW_GEMM_ROWS 3   /* 128x64 row kernel, DSMEM push reduction; KS 1 / 2 / 4 / 8 */
+#define BW_GEMM_TILE 4   /* plain 128xBN tile kernel; BN 32 / 64 / 128 */
+#define BW_GEMM_SIMT 5   /* SIMT kernel (the fp32 validation mode, and bf16 with BW_FLAG_FORCE_SIMT_GEMM) */
+#define BW_GEMM_ROUTE(kernel, param) ((kernel) * 1000 + (param))
+/* Runs one GEMM.  dtype 0: bf16 A / B, C bf16 or fp32 (out_fp32); dtype 1: fp32 A / B / C on the SIMT kernel, as the
+ * fp32 validation mode does.  route 0 = the dispatcher's choice, else BW_GEMM_ROUTE(...) forces that kernel and fails
+ * (BW_ERR_INVALID) if its preconditions do not hold; *route_taken receives the route that ran.  Asynchronous on
+ * `stream` like the engine's launches. */
+int bw_test_gemm(const bw_gemm_desc* desc, int32_t dtype, int32_t route, int32_t* route_taken, void* stream);
+/* Host only (no GPU needed): the route bw_test_gemm(desc, 0, 0, ...) takes, i.e. what the bf16 dispatcher picks for
+ * this argument form.  Pointers are not dereferenced; only whether bias / residual are NULL matters. */
+int bw_test_gemm_route(const bw_gemm_desc* desc, int32_t* route);
 /* Encoder self-attention on qkv [batch*T, 3*64*n_head] bf16 -> out [batch*T, 64*n_head] bf16. impl 0 = tcgen05, 1 = SIMT */
 int bw_attention_bf16(int impl, const void* qkv, void* out, int32_t batch, int32_t T_len, int32_t n_head, void* stream);
 /* Times `iters` launches of the decoder cross-attention kernel on synthetic resident data and returns

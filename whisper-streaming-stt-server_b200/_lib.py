@@ -53,6 +53,21 @@ class DecodeOptsC(C.Structure):
                 ("seed_lo", C.c_uint32), ("seed_hi", C.c_uint32), ("max_candidates", C.c_int32)]
 
 
+class GemmDescC(C.Structure):
+    _fields_ = [("A", C.c_void_p), ("B", C.c_void_p), ("C", C.c_void_p), ("bias", C.c_void_p), ("residual", C.c_void_p)] + [
+        (n, C.c_int32) for n in ("M", "N", "K", "lda", "ldb", "ldc", "ldres", "Z", "a_rows", "b_rows")] + [
+        (n, C.c_int64) for n in ("a_zstride", "b_zstride", "c_zstride", "bias_zstride", "res_zstride")] + [
+        (n, C.c_int32) for n in ("gelu", "out_fp32", "transposed")]
+
+
+# bw_test_gemm routes: BW_GEMM_ROUTE(kernel, param) of include/b200_whisper_hooks.h
+BW_GEMM_PAIR, BW_GEMM_SPLITK, BW_GEMM_ROWS, BW_GEMM_TILE, BW_GEMM_SIMT = 1, 2, 3, 4, 5
+
+
+def gemm_route(kernel: int, param: int = 0) -> int:
+    return kernel * 1000 + param
+
+
 class ResultC(C.Structure):
     _fields_ = [("n_tokens", C.c_int32), ("tokens", C.c_int32 * BW_MAX_TOKENS), ("sum_logprob", C.c_float),
                 ("avg_logprob", C.c_float), ("no_speech_prob", C.c_float), ("n_steps", C.c_int32),
@@ -91,6 +106,8 @@ SIGNATURES = {
     "bw_decode_logits": (C.c_int, [C.c_void_p, c_f32_p, c_i32_p, C.c_int32, c_f32_p]),
     "bw_gemm_bf16": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "bw_test_gemm": (C.c_int, [C.POINTER(GemmDescC), C.c_int32, C.c_int32, c_i32_p, C.c_void_p]),
+    "bw_test_gemm_route": (C.c_int, [C.POINTER(GemmDescC), c_i32_p]),
     "bw_attention_bf16": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "bw_bench_cross_attention": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, c_f32_p, C.POINTER(C.c_double)]),
     "bw_bench_encoder": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, c_f32_p, C.POINTER(C.c_double)]),

@@ -43,8 +43,23 @@ struct GemmArgs {
   float ln_eps = 1e-5f;
 };
 
-// bf16 inputs, fp32 accumulate, tcgen05.mma + TMEM + TMA. Throws on CUDA errors.
+// The kernel a GEMM runs on and its parameter: K split of the cluster split-K and row kernels (1 = the unsplit row
+// kernel), tile width BN of the plain tile kernel, 0 for the pair and SIMT kernels.
+enum class GemmKernel : int { none = 0, pair = 1, splitk = 2, rows = 3, tile = 4, simt = 5 };
+struct GemmRoute {
+  GemmKernel kernel = GemmKernel::none;
+  int param = 0;
+};
+
+// bf16 inputs, fp32 accumulate, tcgen05.mma + TMEM + TMA. Throws on CUDA errors.  Same as
+// gemm_tc_launch(g, gemm_tc_choose(g), stream).
 void gemm_tc_bf16(const GemmArgs& g, cudaStream_t stream);
+// The tcgen05 kernel gemm_tc_bf16 runs for `g`: host only (shape, operand strides and the B200W_* switches).
+GemmRoute gemm_tc_choose(const GemmArgs& g);
+// Why `r` cannot run `g` (nullptr: it can).  The dispatcher only ever picks routes that can.
+const char* gemm_tc_route_error(const GemmArgs& g, GemmRoute r);
+// Runs `g` on route `r`; throws std::invalid_argument if gemm_tc_route_error(g, r) says it cannot.
+void gemm_tc_launch(const GemmArgs& g, GemmRoute r, cudaStream_t stream);
 // Row GEMM of the decoder step (M = live hypotheses): always the push-reduced split-K kernel, any M (more waves for
 // many rows).  The only kernel that understands the LayerNorm-fusion fields of GemmArgs.  N % 64 == 0 required.
 void gemm_tc_rows(const GemmArgs& g, cudaStream_t stream);

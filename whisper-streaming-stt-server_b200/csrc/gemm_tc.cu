@@ -1243,9 +1243,7 @@ void gemm_tc_rows(const GemmArgs& g, cudaStream_t stream) {
   return launch_rows<2>(g, stream);
 }
 
-void gemm_tc_bf16(const GemmArgs& g, cudaStream_t stream) {
-  BW_CHECK(g.M > 0 && g.N > 0 && g.K > 0 && g.Z > 0, "empty GEMM");
-  BW_CHECK(!g.xb_out && !g.ln_stats_out && !g.ln_stats_in, "LayerNorm-fusion fields are only understood by gemm_tc_rows");
+GemmRoute gemm_tc_choose(const GemmArgs& g) {
   // Tile choice: 128x256 (fewer smem bytes per MMA) when it still fills the 148 SMs, else
   // 128x128 with two CTAs per SM; tiny N (swap-AB decode) uses the narrowest tile that covers it.
   const long long mt = (g.M + BM - 1) / BM;
@@ -1253,7 +1251,7 @@ void gemm_tc_bf16(const GemmArgs& g, cudaStream_t stream) {
     // enough 256x256 pair tiles to fill the 74 SM pairs -> persistent cta_group::2 kernel
     static const bool no_pair = getenv("B200W_NO_PAIR") != nullptr;
     const long long pair_tiles = (long long)((g.M + 255) / 256) * ((g.N + 255) / 256) * g.Z;
-    if (!no_pair && !g.transposed && !g.accumulate && pair_tiles >= 60 && g.N >= 256) return launch_pair(g, stream);
+    if (!no_pair && !g.transposed && !g.accumulate && pair_tiles >= 60 && g.N >= 256) return {GemmKernel::pair, 0};
   }
   if (!g.accumulate && g.N > 64 && g.ksplit >= 0) {
     // too few 128x128 tiles for 148 SMs -> split K over a cluster (DSMEM reduction, full epilogue)
@@ -1268,26 +1266,73 @@ void gemm_tc_bf16(const GemmArgs& g, cudaStream_t stream) {
       const long long tiles64 = mt * ((g.N + R_BN - 1) / R_BN) * g.Z;
       int ks = 8;
       while (ks > 2 && (tiles64 * ks > (ks == 8 ? 256 : 288) || total_kb < 2 * ks)) ks >>= 1;
-      if (tiles64 * ks <= 288 && total_kb >= ks) {
-        if (ks == 8) return launch_rows<8>(g, stream);
-        if (ks == 4) return launch_rows<4>(g, stream);
-        return launch_rows<2>(g, stream);
-      }
+      if (tiles64 * ks <= 288 && total_kb >= ks) return {GemmKernel::rows, ks};
     }
     if (tiles < 120 && total_kb >= 4 && !no_splitk) {
       int ks = 8;
       while (ks > 2 && (tiles * ks > 640 || total_kb < 2 * ks)) ks >>= 1;
-      if (ks == 8) return launch_splitk<8>(g, stream);
-      if (ks == 4) return launch_splitk<4>(g, stream);
-      return launch_splitk<2>(g, stream);
+      return {GemmKernel::splitk, ks};
     }
   }
-  if (g.N <= 32) return launch<32, 5, 2>(g, stream);
-  if (g.N <= 64) return launch<64, 4, 2>(g, stream);
-  (void)mt;
+  if (g.N <= 32) return {GemmKernel::tile, 32};
+  if (g.N <= 64) return {GemmKernel::tile, 64};
   // 128x128 with two CTAs per SM: one CTA's epilogue overlaps the other's main loop.  (A 128x256 / 1 CTA
   // variant measured slower here -- profiles/r1a_summary.txt; large GEMMs take the persistent pair kernel above.)
-  return launch<128, 3, 2>(g, stream);
+  return {GemmKernel::tile, 128};
+}
+
+const char* gemm_tc_route_error(const GemmArgs& g, GemmRoute r) {
+  const int total_kb = (g.K + BK - 1) / BK;
+  switch (r.kernel) {
+    case GemmKernel::pair:
+      if (r.param != 0) return "the pair kernel takes no parameter";
+      if (g.transposed || g.accumulate) return "the pair kernel has no transposed or accumulating epilogue";
+      if (g.N < 256) return "the pair kernel needs N >= 256";
+      return nullptr;
+    case GemmKernel::splitk:
+      if (r.param != 2 && r.param != 4 && r.param != 8) return "cluster split-K runs KS = 2, 4 or 8";
+      if (g.accumulate) return "cluster split-K has no accumulating epilogue";
+      if (total_kb < r.param) return "cluster split-K needs at least KS blocks of 64 along K";
+      return nullptr;
+    case GemmKernel::rows:
+      if (r.param != 1 && r.param != 2 && r.param != 4 && r.param != 8) return "the row kernel runs KS = 1, 2, 4 or 8";
+      if (g.transposed || g.accumulate) return "the row kernel has no transposed or accumulating epilogue";
+      if ((g.N % 4) != 0 || (g.ldc % 4) != 0 || (g.residual && (g.ldres % 4) != 0) || (g.bias && (g.bias_zstride % 4) != 0))
+        return "the row kernel needs N, ldc, ldres and bias_zstride % 4 == 0";
+      if (total_kb < r.param) return "the row kernel needs at least KS blocks of 64 along K";
+      return nullptr;
+    case GemmKernel::tile:
+      if (r.param != 32 && r.param != 64 && r.param != 128) return "the tile kernel runs BN = 32, 64 or 128";
+      return nullptr;
+    default:
+      return "not a tcgen05 route";
+  }
+}
+
+void gemm_tc_launch(const GemmArgs& g, GemmRoute r, cudaStream_t stream) {
+  if (const char* why = gemm_tc_route_error(g, r)) throw std::invalid_argument(why);
+  switch (r.kernel) {
+    case GemmKernel::pair: return launch_pair(g, stream);
+    case GemmKernel::splitk:
+      if (r.param == 8) return launch_splitk<8>(g, stream);
+      if (r.param == 4) return launch_splitk<4>(g, stream);
+      return launch_splitk<2>(g, stream);
+    case GemmKernel::rows:
+      if (r.param == 8) return launch_rows<8>(g, stream);
+      if (r.param == 4) return launch_rows<4>(g, stream);
+      if (r.param == 2) return launch_rows<2>(g, stream);
+      return launch_rows<1>(g, stream);
+    default:
+      if (r.param == 32) return launch<32, 5, 2>(g, stream);
+      if (r.param == 64) return launch<64, 4, 2>(g, stream);
+      return launch<128, 3, 2>(g, stream);
+  }
+}
+
+void gemm_tc_bf16(const GemmArgs& g, cudaStream_t stream) {
+  BW_CHECK(g.M > 0 && g.N > 0 && g.K > 0 && g.Z > 0, "empty GEMM");
+  BW_CHECK(!g.xb_out && !g.ln_stats_out && !g.ln_stats_in, "LayerNorm-fusion fields are only understood by gemm_tc_rows");
+  gemm_tc_launch(g, gemm_tc_choose(g), stream);
 }
 
 }  // namespace bw

@@ -23,6 +23,60 @@ int bw_gemm_bf16(int impl, const void* A, const void* B, void* C, const float* b
   BW_API_END
 }
 
+namespace {
+GemmArgs gemm_args_of(const bw_gemm_desc* d) {
+  BW_CHECK(d, "null descriptor");
+  BW_CHECK(d->M > 0 && d->N > 0 && d->K > 0 && d->Z > 0, "empty GEMM");
+  BW_CHECK(d->lda >= d->K && d->ldb >= d->K && d->ldc >= (d->transposed ? d->M : d->N), "leading dimension too small");
+  BW_CHECK(!d->residual || d->ldres >= (d->transposed ? d->M : d->N), "residual leading dimension too small");
+  BW_CHECK((d->a_rows == 0 || d->a_rows >= d->M) && (d->b_rows == 0 || d->b_rows >= d->N), "a_rows / b_rows below M / N");
+  BW_CHECK(d->a_zstride >= 0 && d->b_zstride >= 0 && d->c_zstride >= 0 && d->bias_zstride >= 0 && d->res_zstride >= 0,
+           "negative batch stride");
+  GemmArgs g;
+  g.A = d->A; g.B = d->B; g.C = d->C; g.bias = d->bias; g.residual = d->residual;
+  g.M = d->M; g.N = d->N; g.K = d->K;
+  g.lda = d->lda; g.ldb = d->ldb; g.ldc = d->ldc; g.ldres = d->ldres;
+  g.Z = d->Z; g.a_rows = d->a_rows; g.b_rows = d->b_rows;
+  g.a_zstride = d->a_zstride; g.b_zstride = d->b_zstride; g.c_zstride = d->c_zstride;
+  g.bias_zstride = d->bias_zstride; g.res_zstride = d->res_zstride;
+  g.gelu = d->gelu != 0; g.out_fp32 = d->out_fp32 != 0; g.transposed = d->transposed != 0;
+  return g;
+}
+int route_code(GemmRoute r) { return BW_GEMM_ROUTE((int)r.kernel, r.param); }
+}  // namespace
+
+int bw_test_gemm(const bw_gemm_desc* desc, int32_t dtype, int32_t route, int32_t* route_taken, void* stream) {
+  BW_API_BEGIN
+  BW_CHECK(route_taken, "null argument");
+  const GemmArgs g = gemm_args_of(desc);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const GemmRoute simt{GemmKernel::simt, 0};
+  if (dtype == 1) {
+    BW_CHECK(route == 0 || route == route_code(simt), "the fp32 GEMM runs on the SIMT kernel only");
+    BW_CHECK(g.out_fp32, "the fp32 GEMM writes fp32");
+    gemm_simt<float>(g, st);
+    *route_taken = route_code(simt);
+  } else {
+    BW_CHECK(dtype == 0, "dtype: 0 bf16, 1 fp32");
+    if (route == route_code(simt)) {
+      gemm_simt<bf16>(g, st);
+      *route_taken = route;
+    } else {
+      const GemmRoute r = route == 0 ? gemm_tc_choose(g) : GemmRoute{(GemmKernel)(route / 1000), route % 1000};
+      gemm_tc_launch(g, r, st);
+      *route_taken = route_code(r);
+    }
+  }
+  BW_API_END
+}
+
+int bw_test_gemm_route(const bw_gemm_desc* desc, int32_t* route) {
+  BW_API_BEGIN
+  BW_CHECK(route, "null argument");
+  *route = route_code(gemm_tc_choose(gemm_args_of(desc)));
+  BW_API_END
+}
+
 // Test hook for the decoder LayerNorm fusion: a producer row GEMM (x = res + A.Wp^T + bp, which also leaves bf16(x)
 // and the LayerNorm partials) followed by a consumer row GEMM (out = [gelu](LayerNorm(x).Wc^T + bc) with the
 // LayerNorm folded into Wc).  If A is null the producer is skipped and x = res goes through rows_ln_partials (the
