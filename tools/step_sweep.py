@@ -14,7 +14,6 @@ shapes = ((1, 1), (8, 1), (32, 1), (64, 1), (128, 1), (1, 5), (16, 5), (64, 5))
 if os.environ.get("SWEEP_SHAPES"):
     shapes = tuple(tuple(int(v) for v in s.split("x")) for s in os.environ["SWEEP_SHAPES"].split(","))
 ctxs = tuple(int(v) for v in os.environ.get("SWEEP_CTX", "20,100,200").split(","))
-mode += "".join(f" {k[6:]}={os.environ[k]}" for k in ("B200W_GROUPS",) if os.environ.get(k))
 for seg, grp in shapes:
     for ctx in ctxs:
         eng.bench_decoder_step(seg, grp, ctx, 4)  # the shape's CUDA graph is captured at its third sighting: not in the timed run

@@ -232,26 +232,24 @@ int bw_engine_finalize(bw_engine* e) {
   e->enc_out.alloc((size_t)Be * 1500 * dm * ts);
   // decoder activations
   const size_t R = e->R_max, LR = e->LR_max;
-  for (int gi = 0; gi < kMaxGroups; ++gi) {
-    DecGroup& G = e->grp[gi];
-    BW_CUDA(cudaStreamCreateWithFlags(&G.stream, cudaStreamNonBlocking));
-    G.d_x.alloc(R * dm * 4);
-    G.d_xn.alloc(R * dm * ts); G.d_qkv.alloc(R * 3 * dm * 4); G.d_att.alloc(R * dm * ts); G.d_q.alloc(R * dm * 4);
-    G.d_h.alloc(R * 4 * dm * ts); G.d_lnrows.alloc(LR * dm * ts);
-    if (e->fuse_ln) {
-      G.d_xb.alloc(R * dm * 2);
-      G.d_lnst.alloc(R * (dm / 64) * sizeof(float2));
-      BW_CUDA(cudaMemset(G.d_xb.p, 0, G.d_xb.bytes));
-      BW_CUDA(cudaMemset(G.d_lnst.p, 0, G.d_lnst.bytes));
-    }
-    G.d_pospage.alloc(R * (size_t)d.n_text_ctx * 4);
-    BW_CUDA(cudaMemset(G.d_pospage.p, 0, G.d_pospage.bytes));
-    G.d_logits.alloc(LR * (size_t)d.n_vocab * 4);
-    G.d_ws.alloc(dec_cross_workspace_floats((int)R, d.n_text_head) * 4);
-    G.d_cand_tok.alloc(LR * kMaxCand * 4); G.d_cand_lp.alloc(LR * kMaxCand * 4);
-    // rows past the live count are read (and discarded) by the GEMMs' TMA boxes: keep them finite
-    for (DevBuf* b : {&G.d_xn, &G.d_qkv, &G.d_att, &G.d_q, &G.d_h, &G.d_lnrows}) BW_CUDA(cudaMemset(b->p, 0, b->bytes));
+  DecWorkspace& W = e->dec;
+  BW_CUDA(cudaStreamCreateWithFlags(&W.stream, cudaStreamNonBlocking));
+  W.d_x.alloc(R * dm * 4);
+  W.d_xn.alloc(R * dm * ts); W.d_qkv.alloc(R * 3 * dm * 4); W.d_att.alloc(R * dm * ts); W.d_q.alloc(R * dm * 4);
+  W.d_h.alloc(R * 4 * dm * ts); W.d_lnrows.alloc(LR * dm * ts);
+  if (e->fuse_ln) {
+    W.d_xb.alloc(R * dm * 2);
+    W.d_lnst.alloc(R * (dm / 64) * sizeof(float2));
+    BW_CUDA(cudaMemset(W.d_xb.p, 0, W.d_xb.bytes));
+    BW_CUDA(cudaMemset(W.d_lnst.p, 0, W.d_lnst.bytes));
   }
+  W.d_pospage.alloc(R * (size_t)d.n_text_ctx * 4);
+  BW_CUDA(cudaMemset(W.d_pospage.p, 0, W.d_pospage.bytes));
+  W.d_logits.alloc(LR * (size_t)d.n_vocab * 4);
+  W.d_ws.alloc(dec_cross_workspace_floats((int)R, d.n_text_head) * 4);
+  W.d_cand_tok.alloc(LR * kMaxCand * 4); W.d_cand_lp.alloc(LR * kMaxCand * 4);
+  // rows past the live count are read (and discarded) by the GEMMs' TMA boxes: keep them finite
+  for (DevBuf* b : {&W.d_xn, &W.d_qkv, &W.d_att, &W.d_q, &W.d_h, &W.d_lnrows}) BW_CUDA(cudaMemset(b->p, 0, b->bytes));
   e->d_lang_probs.alloc(128 * 4); e->d_lang_arg.alloc(4);
   BW_CUDA(cudaMemset(e->self_pool.p, 0, e->self_pool.bytes));
   // decoder state
@@ -284,15 +282,12 @@ int bw_engine_finalize(bw_engine* e) {
     ss.anc[0] = e->st_anc0.as<unsigned char>(); ss.anc[1] = e->st_anc1.as<unsigned char>();
     rs.tok = e->st_tok.as<int>(); rs.parent = e->st_parent.as<unsigned char>();
   }
-  // control blocks (one per group) + admission records
+  // decoder-step control block + admission records
   {
-    Ctl probe;
-    probe.layout(nullptr, e->R_max, e->LR_max, Q);
-    e->ctrl_ints = probe.total;
-    for (int gi = 0; gi < kMaxGroups; ++gi) {
-      BW_CUDA(cudaMallocHost(reinterpret_cast<void**>(&e->grp[gi].h_ctrl), e->ctrl_ints * 4));
-      e->grp[gi].d_ctrl.alloc(e->ctrl_ints * 4);
-    }
+    W.ctl.layout(nullptr, e->R_max, e->LR_max, Q);  // sizes only
+    BW_CUDA(cudaMallocHost(reinterpret_cast<void**>(&W.h_ctrl), W.ctl.total * 4));
+    W.ctl.layout(W.h_ctrl, e->R_max, e->LR_max, Q);
+    W.d_ctrl.alloc(W.ctl.total * 4);
     BW_CUDA(cudaMallocHost(reinterpret_cast<void**>(&e->h_init), (size_t)Q * kInitRecInts * 4));
     e->d_init.alloc((size_t)Q * kInitRecInts * 4);
     BW_CUDA(cudaMallocHost(reinterpret_cast<void**>(&e->h_flags), e->step_out_bytes));
@@ -340,11 +335,9 @@ int bw_engine_destroy(bw_engine* e) {
   cudaSetDevice(e->device);
   cudaDeviceSynchronize();
   for (auto& b : e->call_pool) { cudaFree(b.pcm); cudaFree(b.logmel); cudaFree(b.gmax); }
-  for (auto& G : e->grp) {
-    for (auto& kv : G.graphs) if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
-    if (G.h_ctrl) cudaFreeHost(G.h_ctrl);
-    if (G.stream) cudaStreamDestroy(G.stream);
-  }
+  for (auto& kv : e->dec.graphs) if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
+  if (e->dec.h_ctrl) cudaFreeHost(e->dec.h_ctrl);
+  if (e->dec.stream) cudaStreamDestroy(e->dec.stream);
   if (e->h_init) cudaFreeHost(e->h_init);
   if (e->h_flags) cudaFreeHost(e->h_flags);
   if (e->h_fin) cudaFreeHost(e->h_fin);

@@ -207,12 +207,8 @@ struct Impl {
     gemm(g);
   }
 
-  // ---- one decoder step over `R` rows; control arrays already on the device ----
-  struct StepCtl {
-    int R = 0, n_groups = 0, max_group_rows = 1, n_lrows = 0, max_ctx = 0;
-    const int *row_seq, *row_pos, *row_tok, *row_bpos, *row_page, *grp_first, *grp_n, *grp_x, *lrow_src;
-  };
-  SelfKV self_kv(const DecGroup& G) const {
+  // ---- one decoder step over the rows of e->dec.ctl; control block already on the device ----
+  SelfKV self_kv() const {
     const auto& d = D();
     SelfKV skv;
     skv.pool = e->self_pool.p;
@@ -220,25 +216,27 @@ struct Impl {
     skv.n_ctx = d.n_text_ctx; skv.n_blocks = e->n_blocks; skv.n_units = e->S;
     skv.page_table = e->d_page_table.as<int>();
     skv.seq_first = e->ss.seq_first; skv.anc = e->ss.anc[e->anc_cur];
-    skv.pospage = G.d_pospage.as<int>();
+    skv.pospage = e->dec.d_pospage.as<int>();
     return skv;
   }
-  void decoder_layers(const StepCtl& c, DecGroup& G) const {
+  void decoder_layers() const {
     static const bool use_pdl = getenv("B200W_NO_PDL") == nullptr;
     PdlScope pdl(use_pdl && !std::is_same<T, float>::value);
     const auto& d = D();
     const int dm = d.n_text_state, L = d.n_text_layer, H = d.n_text_head;
     cudaStream_t st = stream;
+    const DecWorkspace& G = e->dec;
+    const Ctl& c = G.ctl;
     DecRows rows;
-    rows.n_rows = c.R; rows.row_seq = c.row_seq; rows.row_pos = c.row_pos; rows.row_tok = c.row_tok; rows.row_bpos = c.row_bpos;
-    rows.row_page = c.row_page; rows.max_ctx = c.max_ctx;
+    rows.n_rows = c.R; rows.row_seq = G.dev(c.row_seq); rows.row_pos = G.dev(c.row_pos); rows.row_tok = G.dev(c.row_tok);
+    rows.row_bpos = G.dev(c.row_bpos); rows.row_page = G.dev(c.row_page); rows.max_ctx = c.max_ctx;
     float* x = G.d_x.as<float>();
     if constexpr (std::is_same<T, bf16>::value) {
-      if (e->fuse_ln) return decoder_layers_fused(c, G, rows);
+      if (e->fuse_ln) return decoder_layers_fused(rows);
     }
     dec_embed<T>(rows, e->ss.next_tok, reinterpret_cast<const T*>(e->w.tok_emb), reinterpret_cast<const T*>(e->w.dec_pos), x, dm,
                  e->d_page_table.as<int>(), e->n_blocks, st);
-    const SelfKV skv = self_kv(G);
+    const SelfKV skv = self_kv();
     dec_self_pospage(rows, skv, H, st);
     CrossKV xkv;
     xkv.cache = e->cross_cache.p; xkv.slot_stride = (long long)L * d.n_audio_ctx * 2 * dm; xkv.T_enc = d.n_audio_ctx;
@@ -252,7 +250,7 @@ struct Impl {
       linear_rows(G.d_att.as<T>(), c.R, Ra, w.wo, dm, dm, w.bo, x, x, false, true);
       layernorm<T>(x, w.lnx_g, w.lnx_b, G.d_xn.as<T>(), c.R, dm, st);
       linear_rows(G.d_xn.as<T>(), c.R, Ra, w.wq_x, dm, dm, w.bq_x, nullptr, G.d_q.p, false, true);
-      dec_cross_attention<T>(c.grp_first, c.grp_n, c.grp_x, c.n_groups, c.max_group_rows, c.R, G.d_q.as<float>(), xkv, l, dm, H,
+      dec_cross_attention<T>(G.dev(c.grp_first), G.dev(c.grp_n), G.dev(c.grp_x), c.NG, c.max_grp, c.R, G.d_q.as<float>(), xkv, l, dm, H,
                              G.d_att.as<T>(), G.d_ws.as<float>(), st);
       linear_rows(G.d_att.as<T>(), c.R, Ra, w.wo_x, dm, dm, w.bo_x, x, x, false, true);
       layernorm<T>(x, w.ln2_g, w.ln2_b, G.d_xn.as<T>(), c.R, dm, st);
@@ -260,8 +258,8 @@ struct Impl {
       linear_rows(G.d_h.as<T>(), c.R, Ra, w.w2, dm, 4 * dm, w.b2, x, x, false, true);
     }
     // final LayerNorm only on the rows whose logits are needed, then the tied-embedding projection
-    layernorm_gather<T>(x, c.lrow_src, e->w.ln_g, e->w.ln_b, G.d_lnrows.as<T>(), c.n_lrows, dm, st);
-    linear_rows(G.d_lnrows.as<T>(), c.n_lrows, e->LR_max, e->w.tok_emb, d.n_vocab, dm, nullptr, nullptr, G.d_logits.p, false, true);
+    layernorm_gather<T>(x, G.dev(c.lrow_src), e->w.ln_g, e->w.ln_b, G.d_lnrows.as<T>(), c.LR, dm, st);
+    linear_rows(G.d_lnrows.as<T>(), c.LR, e->LR_max, e->w.tok_emb, d.n_vocab, dm, nullptr, nullptr, G.d_logits.p, false, true);
   }
 
   // bf16 tensor-core mode: the three LayerNorms of a block live inside the row GEMMs.  Each GEMM that writes the
@@ -277,16 +275,18 @@ struct Impl {
     g.xb_out = xb_out; g.ln_stats_out = st_out; g.ln_stats_in = st_in; g.ln_c1 = c1;
     gemm_tc_rows(g, stream);
   }
-  void decoder_layers_fused(const StepCtl& c, DecGroup& G, const DecRows& rows) const {
+  void decoder_layers_fused(const DecRows& rows) const {
     const auto& d = D();
     const int dm = d.n_text_state, L = d.n_text_layer, H = d.n_text_head;
     cudaStream_t st = stream;
+    const DecWorkspace& G = e->dec;
+    const Ctl& c = G.ctl;
     float* x = G.d_x.as<float>();
     bf16* xb = G.d_xb.as<bf16>();
     float2* lst = G.d_lnst.as<float2>();
     dec_embed_ln<bf16>(rows, e->ss.next_tok, reinterpret_cast<const bf16*>(e->w.tok_emb), reinterpret_cast<const bf16*>(e->w.dec_pos), x, dm,
                        xb, lst, e->d_page_table.as<int>(), e->n_blocks, st);
-    const SelfKV skv = self_kv(G);
+    const SelfKV skv = self_kv();
     dec_self_pospage(rows, skv, H, st);
     CrossKV xkv;
     xkv.cache = e->cross_cache.p; xkv.slot_stride = (long long)L * d.n_audio_ctx * 2 * dm; xkv.T_enc = d.n_audio_ctx;
@@ -298,14 +298,14 @@ struct Impl {
       dec_self_attention<bf16>(rows, G.d_qkv.as<float>(), skv, l, dm, H, G.d_att.as<bf16>(), st);
       rows_gemm(G.d_att.p, c.R, Ra, w.wo, dm, dm, w.bo, x, x, false, true, xb, lst, nullptr, nullptr);
       rows_gemm(xb, c.R, Ra, w.wq_x, dm, dm, w.c2_qx, nullptr, G.d_q.p, false, true, nullptr, nullptr, lst, w.c1_qx);
-      dec_cross_attention<bf16>(c.grp_first, c.grp_n, c.grp_x, c.n_groups, c.max_group_rows, c.R, G.d_q.as<float>(), xkv, l, dm, H,
+      dec_cross_attention<bf16>(G.dev(c.grp_first), G.dev(c.grp_n), G.dev(c.grp_x), c.NG, c.max_grp, c.R, G.d_q.as<float>(), xkv, l, dm, H,
                                 G.d_att.as<bf16>(), G.d_ws.as<float>(), st);
       rows_gemm(G.d_att.p, c.R, Ra, w.wo_x, dm, dm, w.bo_x, x, x, false, true, xb, lst, nullptr, nullptr);
       rows_gemm(xb, c.R, Ra, w.w1, 4 * dm, dm, w.c2_w1, nullptr, G.d_h.p, true, false, nullptr, nullptr, lst, w.c1_w1);
       rows_gemm(G.d_h.p, c.R, Ra, w.w2, dm, 4 * dm, w.b2, x, x, false, true, xb, lst, nullptr, nullptr);
     }
-    layernorm_gather<bf16>(x, c.lrow_src, e->w.ln_g, e->w.ln_b, G.d_lnrows.as<bf16>(), c.n_lrows, dm, st);
-    linear_rows(G.d_lnrows.as<bf16>(), c.n_lrows, e->LR_max, e->w.tok_emb, d.n_vocab, dm, nullptr, nullptr, G.d_logits.p, false, true);
+    layernorm_gather<bf16>(x, G.dev(c.lrow_src), e->w.ln_g, e->w.ln_b, G.d_lnrows.as<bf16>(), c.LR, dm, st);
+    linear_rows(G.d_lnrows.as<bf16>(), c.LR, e->LR_max, e->w.tok_emb, d.n_vocab, dm, nullptr, nullptr, G.d_logits.p, false, true);
   }
 
   void window_to_A1(const float* logmel, int ld, int n_real, const int* gmax, int seek, int seg, int bi) const {
@@ -507,18 +507,8 @@ void engine_window_to_A1(bw_engine* e, const float* logmel, int ld, int n_real, 
   if (e->fp32) Impl<float>(e).window_to_A1(logmel, ld, n_real, gmax, seek, seg, bi);
   else Impl<bf16>(e).window_to_A1(logmel, ld, n_real, gmax, seek, seg, bi);
 }
-void engine_decoder_layers(bw_engine* e, DecGroup& G, int R, int n_groups, int max_group_rows, int n_lrows, int max_ctx, const int* row_seq,
-                           const int* row_pos, const int* row_tok, const int* row_bpos, const int* row_page, const int* grp_first,
-                           const int* grp_n, const int* grp_x, const int* lrow_src) {
-  if (e->fp32) {
-    Impl<float>::StepCtl c; c.R = R; c.n_groups = n_groups; c.max_group_rows = max_group_rows; c.n_lrows = n_lrows; c.max_ctx = max_ctx;
-    c.row_seq = row_seq; c.row_pos = row_pos; c.row_tok = row_tok; c.row_bpos = row_bpos; c.row_page = row_page; c.grp_first = grp_first; c.grp_n = grp_n; c.grp_x = grp_x; c.lrow_src = lrow_src;
-    Impl<float>(e, G.stream).decoder_layers(c, G);
-  } else {
-    Impl<bf16>::StepCtl c; c.R = R; c.n_groups = n_groups; c.max_group_rows = max_group_rows; c.n_lrows = n_lrows; c.max_ctx = max_ctx;
-    c.row_seq = row_seq; c.row_pos = row_pos; c.row_tok = row_tok; c.row_bpos = row_bpos; c.row_page = row_page; c.grp_first = grp_first; c.grp_n = grp_n; c.grp_x = grp_x; c.lrow_src = lrow_src;
-    Impl<bf16>(e, G.stream).decoder_layers(c, G);
-  }
+void engine_decoder_layers(bw_engine* e) {
+  if (e->fp32) Impl<float>(e, e->dec.stream).decoder_layers(); else Impl<bf16>(e, e->dec.stream).decoder_layers();
 }
 void engine_gather_final(bw_engine* e, const int* list_dev, int n, int blob_bytes, unsigned char* out_dev) {
   if (n <= 0) return;

@@ -71,9 +71,6 @@ struct ModelW {
 
 enum ReqKind { REQ_DECODE = 0, REQ_LANG = 1, REQ_LOGITS = 2 };
 
-// Decoder-step working set of one request group.  The live requests of a step are split into up to kMaxGroups
-// groups that run on their own streams: one group's latency-bound LayerNorm / skinny-GEMM chain executes
-// underneath another group's HBM-bound cross-attention.
 struct StepGraphKey {
   int R, NG, LR, SR, NA, NNS, max_grp, anc, self_chunk;  // self_chunk: the self-attention launch geometry (dec_self_chunk)
   bool operator==(const StepGraphKey& o) const {
@@ -93,9 +90,31 @@ struct StepGraph {
   unsigned long long last_use = 0;
   cudaGraphExec_t exec = nullptr;
 };
-constexpr size_t kMaxStepGraphs = 128;  // per group; least recently used half is dropped beyond this
+constexpr size_t kMaxStepGraphs = 128;  // per engine; least recently used half is dropped beyond this
 
-struct DecGroup {
+// ---- decoder-step control block (ints), mirrored host (pinned) / device ----
+struct Ctl {
+  int *row_seq, *row_pos, *row_tok, *row_bpos, *row_page, *grp_first, *grp_n, *grp_x, *lrow_src, *srow_lrow, *srow_req, *srow_seq, *act_req,
+      *act_first, *act_force, *ns_lrow, *ns_req;
+  int* base = nullptr;
+  size_t total = 0;
+  // fill counters of the step being built
+  int R = 0, NG = 0, LR = 0, SR = 0, NA = 0, NNS = 0, max_grp = 1, max_ctx = 0;
+  void layout(int* b, int Rm, int LRm, int Q) {
+    base = b;
+    int* p = b;
+    auto take = [&](size_t n) { int* r = p; p += n; return r; };
+    row_seq = take(Rm); row_pos = take(Rm); row_tok = take(Rm); row_bpos = take(Rm); row_page = take(Rm);
+    grp_first = take(Rm); grp_n = take(Rm); grp_x = take(Rm);
+    lrow_src = take(LRm); srow_lrow = take(LRm); srow_req = take(LRm); srow_seq = take(LRm);
+    act_req = take(Q); act_first = take(Q); act_force = take(Q); ns_lrow = take(Q); ns_req = take(Q);
+    total = (size_t)(p - b);
+  }
+  void reset() { R = NG = LR = SR = NA = NNS = 0; max_grp = 1; max_ctx = 0; }
+};
+
+// Decoder-step working set: activations, logits, control block and step graphs, with the step's own stream.
+struct DecWorkspace {
   cudaStream_t stream = nullptr;
   // CUDA graphs of the whole decoder step, keyed by its shape: while the set of live requests is unchanged only the
   // control block's CONTENTS change from step to step, so ~360 launches collapse into one cudaGraphLaunch.
@@ -105,8 +124,9 @@ struct DecGroup {
   DevBuf d_xb, d_lnst;  // LayerNorm fusion: bf16 copy of the residual stream, per-row / per-64-column partials
   DevBuf d_pospage;     // [R_max][n_text_ctx] page of (row, position) for the step's self-attention (dec_self_pospage)
   int* h_ctrl = nullptr;  // pinned host copy of the control block
+  Ctl ctl;                // laid out over h_ctrl
+  int* dev(const int* h) const { return d_ctrl.as<int>() + (h - ctl.base); }  // device address of a control array
 };
-constexpr int kMaxGroups = 4;
 
 // polyphase filter bank of one source sample rate (bw_engine_set_resampler)
 struct Resampler {
@@ -220,8 +240,8 @@ struct bw_engine {
   std::atomic<long long> stat_pages_in_use{0}, stat_pages_peak{0};
   // encoder activations
   bw::DevBuf A1, y1, A2, enc_x, enc_xn, enc_qkv, enc_att, enc_h, enc_out;
-  // decoder activations: one working set per request group
-  bw::DecGroup grp[bw::kMaxGroups];
+  // decoder activations
+  bw::DecWorkspace dec;
   bw::DevBuf d_lang_probs, d_lang_arg;
   // decoder state
   bw::DevBuf st_int, st_float, st_anc0, st_anc1, st_tok, st_parent, st_step;  // st_step: [Q] completed | [Q][kMaxBeam] last_src
@@ -231,7 +251,6 @@ struct bw_engine {
   // admission records (init_requests_kernel input)
   bw::DevBuf d_init;
   int* h_init = nullptr;      // pinned
-  size_t ctrl_ints = 0;
   int* h_flags = nullptr;     // pinned copy of st_step: [Q] completed flags, then [Q][kMaxBeam] parent slots (bytes)
   size_t step_out_bytes = 0;
   unsigned char* h_fin = nullptr;  // pinned scratch for finalisation

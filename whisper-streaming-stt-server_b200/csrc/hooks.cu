@@ -199,7 +199,6 @@ int bw_bench_encoder(bw_engine* e, int32_t batch, int32_t iters, float* ms_out, 
 
 namespace {
 // Synthetic resident decode: `n_segments` windows x `n_group` hypotheses, positions [start_len, start_len + n_steps).
-// Same launches, control upload and per-step completion read-back as the scheduler's decode_step().
 // pages of the synthetic decode: hypothesis slot u, block b -> page u * nb + b (the engine is idle: every page is free)
 int synthetic_pages(bw_engine* e, int n_segments, int n_group, int max_len) {
   const int nb = kv_blocks_for(max_len);
@@ -221,12 +220,12 @@ void synthetic_init(bw_engine* e, int n_segments, int n_group, int start_len) {
   engine_init_requests(e, e->d_init.as<int>(), n_segments);
   BW_CUDA(cudaStreamSynchronize(e->stream));
 }
-// same grouping, launches, control upload and per-step completion read-back as the scheduler's decode_step()
-void synthetic_step(bw_engine* e, Ctl* ctls, int n_segments, int n_group, int cur, int nb) {
-  const int ng = choose_groups(n_segments);
-  for (int g = 0; g < ng; ++g) ctls[g].reset();
+// One step: the control block filled as decode_step() fills it for decodes past their prompt, then the control
+// upload, launches and completion read-back of decode_step() itself (enqueue_step, finish_step).
+void synthetic_step(bw_engine* e, int n_segments, int n_group, int cur, int nb) {
+  Ctl& c = e->dec.ctl;
+  c.reset();
   for (int i = 0; i < n_segments; ++i) {
-    Ctl& c = ctls[i % ng];
     c.grp_first[c.NG] = c.R; c.grp_n[c.NG] = n_group; c.grp_x[c.NG] = i; ++c.NG;
     c.max_grp = std::max(c.max_grp, n_group);
     c.max_ctx = std::max(c.max_ctx, cur);
@@ -238,21 +237,9 @@ void synthetic_step(bw_engine* e, Ctl* ctls, int n_segments, int n_group, int cu
       ++c.R; ++c.LR; ++c.SR;
     }
   }
-  for (int g = 0; g < ng; ++g) enqueue_group_step(e, e->grp[g], ctls[g]);
-  if (ng == 1) {
-    BW_CUDA(cudaMemcpyAsync(e->h_flags, e->st_step.p, e->step_out_bytes, cudaMemcpyDeviceToHost, e->grp[0].stream));
-    BW_CUDA(cudaStreamSynchronize(e->grp[0].stream));
-  } else {
-    for (int g = 0; g < ng; ++g) BW_CUDA(cudaStreamSynchronize(e->grp[g].stream));
-    BW_CUDA(cudaMemcpyAsync(e->h_flags, e->st_step.p, e->step_out_bytes, cudaMemcpyDeviceToHost, e->stream));
-    BW_CUDA(cudaStreamSynchronize(e->stream));
-  }
-  e->anc_cur ^= 1;
+  enqueue_step(e);
+  finish_step(e);
 }
-struct SynCtls {
-  Ctl c[kMaxGroups];
-  explicit SynCtls(bw_engine* e) { for (int g = 0; g < kMaxGroups; ++g) c[g].layout(e->grp[g].h_ctrl, e->R_max, e->LR_max, e->Q); }
-};
 }  // namespace
 
 // One full decoder step (all layers + logits + sampling + beam update) over `n_segments` resident
@@ -267,7 +254,6 @@ int bw_bench_decoder_step(bw_engine* e, int32_t n_segments, int32_t n_group, int
   DeviceGuard dg(e->device);
   std::lock_guard<std::mutex> g(e->gpu_mu);
   BW_CHECK(e->live.empty(), "engine busy");
-  SynCtls sc(e);
   fill_cross_cache(e, n_segments);
   BW_CHECK(e->stat_pages_in_use == 0, "engine busy");
   const int nb = synthetic_pages(e, n_segments, n_group, context_len + iters + 2);
@@ -278,10 +264,10 @@ int bw_bench_decoder_step(bw_engine* e, int32_t n_segments, int32_t n_group, int
   }
   synthetic_init(e, n_segments, n_group, context_len);
   int cur = context_len;
-  synthetic_step(e, sc.c, n_segments, n_group, cur++, nb);
-  EvTimer t(e->stream);  // e->stream is idle here and receives the completion read-back of every step
+  synthetic_step(e, n_segments, n_group, cur++, nb);
+  EvTimer t(e->stream);  // e->stream is idle here; every step ends in a host synchronisation with the decoder stream
   t.start();
-  for (int i = 0; i < iters; ++i) synthetic_step(e, sc.c, n_segments, n_group, cur++, nb);
+  for (int i = 0; i < iters; ++i) synthetic_step(e, n_segments, n_group, cur++, nb);
   *ms_out = t.stop_ms() / iters;
   const double ts = e->fp32 ? 4 : 2, d = e->dims.n_text_state, L = e->dims.n_text_layer, V = e->dims.n_vocab;
   const double S = (double)n_segments * n_group;
@@ -314,7 +300,6 @@ int bw_bench_pipeline(bw_engine* e, const float* pcm_host, const int64_t* offset
   BW_CUDA(cudaStreamSynchronize(e->stream));
   BW_CHECK(e->stat_pages_in_use == 0, "engine busy");
   const int nb = synthetic_pages(e, n_segments, n_group, 3 + n_steps + 1);
-  SynCtls sc(e);
   auto frames = [&](int i, int& total, int& n_real, int& seg) {
     total = (int)((lengths[i] + 480000) / 160);
     n_real = (int)std::min<long long>(total, (lengths[i] + 200 + 159) / 160);
@@ -339,7 +324,7 @@ int bw_bench_pipeline(bw_engine* e, const float* pcm_host, const int64_t* offset
     for (int i = 0; i < nb; ++i) engine_cross_kv(e, i, s0 + i);
   }
   synthetic_init(e, n_segments, n_group, 3);
-  for (int i = 0; i < n_steps; ++i) synthetic_step(e, sc.c, n_segments, n_group, 3 + i, nb);
+  for (int i = 0; i < n_steps; ++i) synthetic_step(e, n_segments, n_group, 3 + i, nb);
   *ms_out = t.stop_ms();
   {
     std::lock_guard<std::mutex> cg(e->call_mu);
@@ -391,27 +376,24 @@ int bw_bench_cross_attention(bw_engine* e, int32_t n_segments, int32_t n_group, 
   BW_CHECK(n_segments * n_group <= e->R_max, "too many rows");
   DeviceGuard dg(e->device);
   std::lock_guard<std::mutex> g(e->gpu_mu);
-  SynCtls sc(e);
-  Ctl& ctl = sc.c[0];
-  DecGroup& G = e->grp[0];
+  DecWorkspace& W = e->dec;
+  Ctl& ctl = W.ctl;
   for (int i = 0; i < n_segments; ++i) { ctl.grp_first[i] = i * n_group; ctl.grp_n[i] = n_group; ctl.grp_x[i] = i; }
-  int* dbase = G.d_ctrl.as<int>();
-  auto dev = [&](int* h) { return dbase + (h - ctl.base); };
-  BW_CUDA(cudaMemcpyAsync(dbase, ctl.base, ctl.total * 4, cudaMemcpyHostToDevice, e->stream));
+  BW_CUDA(cudaMemcpyAsync(W.d_ctrl.p, ctl.base, ctl.total * 4, cudaMemcpyHostToDevice, e->stream));
   fill_cross_cache(e, n_segments);
   const auto& d = e->dims;
   const int dm = d.n_text_state, L = d.n_text_layer;
   const int R = n_segments * n_group;
-  fill_random<float>(G.d_q.as<float>(), (long long)R * dm, 0x9ull, 1.f, e->stream);
+  fill_random<float>(W.d_q.as<float>(), (long long)R * dm, 0x9ull, 1.f, e->stream);
   auto run = [&](int layer) {
     CrossKV x; x.cache = e->cross_cache.p; x.slot_stride = (long long)L * d.n_audio_ctx * 2 * dm; x.T_enc = d.n_audio_ctx;
     x.n_slots = e->Q; x.n_layer = L;
     if (e->fp32)
-      dec_cross_attention<float>(dev(ctl.grp_first), dev(ctl.grp_n), dev(ctl.grp_x), n_segments, n_group, R, G.d_q.as<float>(), x, layer, dm,
-                                 d.n_text_head, G.d_att.as<float>(), G.d_ws.as<float>(), e->stream);
+      dec_cross_attention<float>(W.dev(ctl.grp_first), W.dev(ctl.grp_n), W.dev(ctl.grp_x), n_segments, n_group, R, W.d_q.as<float>(), x,
+                                 layer, dm, d.n_text_head, W.d_att.as<float>(), W.d_ws.as<float>(), e->stream);
     else
-      dec_cross_attention<bf16>(dev(ctl.grp_first), dev(ctl.grp_n), dev(ctl.grp_x), n_segments, n_group, R, G.d_q.as<float>(), x, layer, dm,
-                                d.n_text_head, G.d_att.as<bf16>(), G.d_ws.as<float>(), e->stream);
+      dec_cross_attention<bf16>(W.dev(ctl.grp_first), W.dev(ctl.grp_n), W.dev(ctl.grp_x), n_segments, n_group, R, W.d_q.as<float>(), x,
+                                layer, dm, d.n_text_head, W.d_att.as<bf16>(), W.d_ws.as<float>(), e->stream);
   };
   run(0);
   EvTimer t(e->stream);

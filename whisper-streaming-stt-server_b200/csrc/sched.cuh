@@ -18,9 +18,7 @@ void engine_load_tensor(bw_engine* e, const bw_tensor_desc& t);
 void engine_encoder_forward(bw_engine* e, int nb);
 void engine_cross_kv(bw_engine* e, int bi, int q);
 void engine_window_to_A1(bw_engine* e, const float* logmel, int ld, int n_real, const int* gmax, int seek, int seg, int bi);
-void engine_decoder_layers(bw_engine* e, DecGroup& G, int R, int n_groups, int max_group_rows, int n_lrows, int max_ctx, const int* row_seq,
-                           const int* row_pos, const int* row_tok, const int* row_bpos, const int* row_page, const int* grp_first,
-                           const int* grp_n, const int* grp_x, const int* lrow_src);
+void engine_decoder_layers(bw_engine* e);  // the step that e->dec.ctl describes, on e->dec.stream
 void engine_init_requests(bw_engine* e, const int* init_dev, int n);
 void engine_fold_layernorms(bw_engine* e);
 void engine_gather_final(bw_engine* e, const int* list_dev, int n, int blob_bytes, unsigned char* out_dev);
@@ -36,30 +34,11 @@ struct DeviceGuard {
   ~DeviceGuard() { cudaSetDevice(prev); }
 };
 
-// ---- per-group control block (ints), mirrored host (pinned) / device ----
-struct Ctl {
-  int *row_seq, *row_pos, *row_tok, *row_bpos, *row_page, *grp_first, *grp_n, *grp_x, *lrow_src, *srow_lrow, *srow_req, *srow_seq, *act_req,
-      *act_first, *act_force, *ns_lrow, *ns_req;
-  int* base = nullptr;
-  size_t total = 0;
-  // fill counters of the step being built
-  int R = 0, NG = 0, LR = 0, SR = 0, NA = 0, NNS = 0, max_grp = 1, max_ctx = 0;
-  void layout(int* b, int Rm, int LRm, int Q) {
-    base = b;
-    int* p = b;
-    auto take = [&](size_t n) { int* r = p; p += n; return r; };
-    row_seq = take(Rm); row_pos = take(Rm); row_tok = take(Rm); row_bpos = take(Rm); row_page = take(Rm);
-    grp_first = take(Rm); grp_n = take(Rm); grp_x = take(Rm);
-    lrow_src = take(LRm); srow_lrow = take(LRm); srow_req = take(LRm); srow_seq = take(LRm);
-    act_req = take(Q); act_first = take(Q); act_force = take(Q); ns_lrow = take(Q); ns_req = take(Q);
-    total = (size_t)(p - b);
-  }
-  void reset() { R = NG = LR = SR = NA = NNS = 0; max_grp = 1; max_ctx = 0; }
-};
-
 // scheduler.cu
-void enqueue_group_step(bw_engine* e, DecGroup& G, Ctl& c);
-int choose_groups(int n_segments);
+// the decoder step that e->dec.ctl describes (control upload included), a CUDA graph from the third step of its shape
+void enqueue_step(bw_engine* e);
+// completion of the step: the flags and beam parents (st_step) to h_flags, one host synchronisation, anc_cur flipped
+void finish_step(bw_engine* e);
 void scheduler_main(bw_engine* e);
 // self-KV page pool (host free list; scheduler thread / synthetic benches only)
 int kv_blocks_for(int n_tokens);                       // pages one hypothesis needs for n_tokens positions

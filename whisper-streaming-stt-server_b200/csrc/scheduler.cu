@@ -18,80 +18,80 @@ void finish_request(Request* r, int status, const std::string& err) {
   r->cv.notify_all();
 }
 
-// H2D of the control block + the whole decoder step (all layers, logits, filters/top-k, beam update) of one group,
-// enqueued on the group's stream.  No host synchronisation here.
-void enqueue_group_step_eager(bw_engine* e, DecGroup& G, Ctl& c) {
-  int* dbase = G.d_ctrl.as<int>();
-  auto dev = [&](int* h) { return dbase + (h - c.base); };
-  BW_CUDA(cudaMemcpyAsync(dbase, c.base, c.total * 4, cudaMemcpyHostToDevice, G.stream));
-  engine_decoder_layers(e, G, c.R, c.NG, c.max_grp, c.LR, c.max_ctx, dev(c.row_seq), dev(c.row_pos), dev(c.row_tok), dev(c.row_bpos),
-                        dev(c.row_page), dev(c.grp_first), dev(c.grp_n), dev(c.grp_x), dev(c.lrow_src));
-  const float* logits = G.d_logits.as<float>();
+// H2D of the control block + the whole decoder step (all layers, logits, filters/top-k, beam update), enqueued on the
+// decoder stream.  No host synchronisation here.
+void enqueue_step_eager(bw_engine* e) {
+  DecWorkspace& W = e->dec;
+  const Ctl& c = W.ctl;
+  BW_CUDA(cudaMemcpyAsync(W.d_ctrl.p, c.base, c.total * 4, cudaMemcpyHostToDevice, W.stream));
+  engine_decoder_layers(e);
+  const float* logits = W.d_logits.as<float>();
   const int V = e->dims.n_vocab;
   static const bool use_pdl = getenv("B200W_NO_PDL") == nullptr;
   PdlScope pdl(use_pdl && !e->fp32);
-  no_speech_prob(logits, V, V, dev(c.ns_lrow), dev(c.ns_req), c.NNS, e->tt.no_speech, e->rs.no_speech_prob, G.stream);
-  sample_topk(logits, V, V, dev(c.srow_lrow), dev(c.srow_req), dev(c.srow_seq), c.SR, e->tt, e->rs, e->ss, e->anc_cur,
-              G.d_cand_tok.as<int>(), G.d_cand_lp.as<float>(), G.stream);
-  beam_update(dev(c.act_req), dev(c.act_first), dev(c.act_force), c.NA, e->tt, e->rs, e->ss, e->anc_cur, e->dims.n_text_ctx,
-              G.d_cand_tok.as<int>(), G.d_cand_lp.as<float>(), G.stream);
+  no_speech_prob(logits, V, V, W.dev(c.ns_lrow), W.dev(c.ns_req), c.NNS, e->tt.no_speech, e->rs.no_speech_prob, W.stream);
+  sample_topk(logits, V, V, W.dev(c.srow_lrow), W.dev(c.srow_req), W.dev(c.srow_seq), c.SR, e->tt, e->rs, e->ss, e->anc_cur,
+              W.d_cand_tok.as<int>(), W.d_cand_lp.as<float>(), W.stream);
+  beam_update(W.dev(c.act_req), W.dev(c.act_first), W.dev(c.act_force), c.NA, e->tt, e->rs, e->ss, e->anc_cur, e->dims.n_text_ctx,
+              W.d_cand_tok.as<int>(), W.d_cand_lp.as<float>(), W.stream);
 }
 
 
 }  // namespace
 
-void enqueue_group_step(bw_engine* e, DecGroup& G, Ctl& c) {
+void enqueue_step(bw_engine* e) {
+  DecWorkspace& W = e->dec;
+  const Ctl& c = W.ctl;
   if (c.R == 0) return;
   e->stat_h2d += (long long)c.total * 4;
   static const bool use_graphs = getenv("B200W_NO_GRAPH") == nullptr;
-  if (!use_graphs) return enqueue_group_step_eager(e, G, c);
+  if (!use_graphs) return enqueue_step_eager(e);
   const StepGraphKey key{c.R, c.NG, c.LR, c.SR, c.NA, c.NNS, c.max_grp, e->anc_cur, dec_self_chunk(c.max_ctx)};
-  StepGraph& sg = G.graphs[key];
-  sg.last_use = ++G.graph_clock;
+  StepGraph& sg = W.graphs[key];
+  sg.last_use = ++W.graph_clock;
   if (sg.exec) {
-    BW_CUDA(cudaGraphLaunch(sg.exec, G.stream));
+    BW_CUDA(cudaGraphLaunch(sg.exec, W.stream));
     return;
   }
-  if (++sg.seen < 3) return enqueue_group_step_eager(e, G, c);  // early sightings also warm every lazy initialisation
+  if (++sg.seen < 3) return enqueue_step_eager(e);  // early sightings also warm every lazy initialisation
   // third sighting of this shape: it is stable enough to pay for a capture (the launch sequence depends only on the key)
   cudaGraph_t graph = nullptr;
-  BW_CUDA(cudaStreamBeginCapture(G.stream, cudaStreamCaptureModeThreadLocal));
+  BW_CUDA(cudaStreamBeginCapture(W.stream, cudaStreamCaptureModeThreadLocal));
   try {
-    enqueue_group_step_eager(e, G, c);
+    enqueue_step_eager(e);
   } catch (...) {
-    cudaStreamEndCapture(G.stream, &graph);
+    cudaStreamEndCapture(W.stream, &graph);
     if (graph) cudaGraphDestroy(graph);
     throw;
   }
-  BW_CUDA(cudaStreamEndCapture(G.stream, &graph));
+  BW_CUDA(cudaStreamEndCapture(W.stream, &graph));
   cudaGraphExec_t exec = nullptr;
   const cudaError_t st = cudaGraphInstantiate(&exec, graph, 0);
   cudaGraphDestroy(graph);
   if (st != cudaSuccess) throw CudaError(std::string("cudaGraphInstantiate -> ") + cudaGetErrorString(st));
   sg.exec = exec;
-  sg.last_use = ++G.graph_clock;
-  BW_CUDA(cudaGraphLaunch(exec, G.stream));
-  if (G.graphs.size() > kMaxStepGraphs) {
+  sg.last_use = ++W.graph_clock;
+  BW_CUDA(cudaGraphLaunch(exec, W.stream));
+  if (W.graphs.size() > kMaxStepGraphs) {
     // bound the cache (shapes churn while requests come and go): drop the least recently used half, entries included.
     // `sg` is not touched after this point (erase invalidates references to the erased nodes only, but be explicit).
     std::vector<std::pair<unsigned long long, StepGraphKey>> order;
-    order.reserve(G.graphs.size());
-    for (auto& kv : G.graphs) order.emplace_back(kv.second.last_use, kv.first);
+    order.reserve(W.graphs.size());
+    for (auto& kv : W.graphs) order.emplace_back(kv.second.last_use, kv.first);
     std::sort(order.begin(), order.end(), [](const auto& a, const auto& b) { return a.first < b.first; });
-    BW_CUDA(cudaStreamSynchronize(G.stream));  // no captured graph of the evicted half may still be running
+    BW_CUDA(cudaStreamSynchronize(W.stream));  // no captured graph of the evicted half may still be running
     for (size_t i = 0; i < order.size() / 2; ++i) {
-      auto it = G.graphs.find(order[i].second);
+      auto it = W.graphs.find(order[i].second);
       if (it->second.exec) cudaGraphExecDestroy(it->second.exec);
-      G.graphs.erase(it);
+      W.graphs.erase(it);
     }
   }
 }
 
-int choose_groups(int n_segments) {
-  static const int forced = getenv("B200W_GROUPS") ? atoi(getenv("B200W_GROUPS")) : 0;
-  if (forced > 0) return std::min(forced, (int)kMaxGroups);
-  (void)n_segments;
-  return 1;  // measured: extra groups re-stream the weights and lengthen the step (profiles/r1_notes.md)
+void finish_step(bw_engine* e) {
+  BW_CUDA(cudaMemcpyAsync(e->h_flags, e->st_step.p, e->step_out_bytes, cudaMemcpyDeviceToHost, e->dec.stream));
+  BW_CUDA(cudaStreamSynchronize(e->dec.stream));
+  e->anc_cur ^= 1;
 }
 
 // ---- self-KV page pool -------------------------------------------------------------------------------------------
@@ -364,16 +364,14 @@ int forced_token(const Request* r) {
   return (r->steps < (int)r->forced.size()) ? r->forced[r->steps] : -1;
 }
 
-void decode_step(bw_engine* e, Ctl* ctls) {
+void decode_step(bw_engine* e) {
   const auto& d = e->dims;
-  struct Special { Request* r; int grp; int lrow0; int n; };
+  struct Special { Request* r; int lrow0; int n; };
   std::vector<Special> lang_reqs, logit_reqs, forced_reqs;
-  const int ng = choose_groups((int)e->live.size());
-  for (int g = 0; g < ng; ++g) ctls[g].reset();
+  DecWorkspace& W = e->dec;
+  Ctl& ctl = W.ctl;
+  ctl.reset();
   for (Request* r : e->live) {
-    int gi = 0;  // least-loaded group (rows)
-    for (int g = 1; g < ng; ++g) if (ctls[g].R < ctls[gi].R) gi = g;
-    Ctl& ctl = ctls[gi];
     int &R = ctl.R, &NG = ctl.NG, &LR = ctl.LR, &SR = ctl.SR, &NA = ctl.NA, &NNS = ctl.NNS, &max_grp = ctl.max_grp;
     if (!r->prefilled) {
       const int n_init = (int)r->initial.size();
@@ -394,10 +392,10 @@ void decode_step(bw_engine* e, Ctl* ctls) {
       }
       if (r->kind == REQ_LANG) {
         ctl.lrow_src[LR] = row0;
-        lang_reqs.push_back({r, gi, LR, 1});
+        lang_reqs.push_back({r, LR, 1});
         ++LR;
       } else if (r->kind == REQ_LOGITS) {
-        logit_reqs.push_back({r, gi, LR, n_init});
+        logit_reqs.push_back({r, LR, n_init});
         for (int t = 0; t < n_init; ++t) ctl.lrow_src[LR++] = row0 + t;
       } else {
         const int last_row = row0 + n_init - 1;
@@ -410,7 +408,7 @@ void decode_step(bw_engine* e, Ctl* ctls) {
         ctl.ns_lrow[NNS] = sot_lrow; ctl.ns_req[NNS] = r->q; ++NNS;
         ctl.act_req[NA] = r->q; ctl.act_first[NA] = SR; ctl.act_force[NA] = forced_token(r); ++NA;
         ctl.srow_lrow[SR] = LR; ctl.srow_req[SR] = r->q; ctl.srow_seq[SR] = r->first_seq; ++SR;
-        if (r->step_logits_out) forced_reqs.push_back({r, gi, LR, 1});
+        if (r->step_logits_out) forced_reqs.push_back({r, LR, 1});
         ++LR;
       }
     } else {
@@ -419,7 +417,7 @@ void decode_step(bw_engine* e, Ctl* ctls) {
       ctl.max_ctx = std::max(ctl.max_ctx, r->cur_len);
       ++NG;
       ctl.act_req[NA] = r->q; ctl.act_first[NA] = SR; ctl.act_force[NA] = forced_token(r); ++NA;
-      if (r->step_logits_out) forced_reqs.push_back({r, gi, LR, 1});
+      if (r->step_logits_out) forced_reqs.push_back({r, LR, 1});
       for (int j = 0; j < r->G; ++j) {
         ctl.row_seq[R] = r->first_seq + j; ctl.row_pos[R] = r->cur_len - 1; ctl.row_tok[R] = -1; ctl.row_bpos[R] = r->cur_len - 1;
         ctl.row_page[R] = kv_page_of(e, r, j, (r->cur_len - 1) / kPageTokens);  // slot j writes position cur_len - 1
@@ -430,39 +428,28 @@ void decode_step(bw_engine* e, Ctl* ctls) {
       }
     }
   }
-  int total_rows = 0;
-  for (int g = 0; g < ng; ++g) { enqueue_group_step(e, e->grp[g], ctls[g]); total_rows += ctls[g].R; }
+  enqueue_step(e);
   const int V = d.n_vocab;
   for (auto& s : lang_reqs) {
-    DecGroup& G = e->grp[s.grp];
-    language_probs(G.d_logits.as<float>() + (size_t)s.lrow0 * V, V, e->tt.first_language_token, e->tt.num_languages,
-                   e->d_lang_probs.as<float>(), e->d_lang_arg.as<int>(), G.stream);
-    BW_CUDA(cudaMemcpyAsync(s.r->lang_out->probs, e->d_lang_probs.p, (size_t)e->tt.num_languages * 4, cudaMemcpyDeviceToHost, G.stream));
-    BW_CUDA(cudaMemcpyAsync(&s.r->lang_out->language_token, e->d_lang_arg.p, 4, cudaMemcpyDeviceToHost, G.stream));
-    BW_CUDA(cudaStreamSynchronize(G.stream));
+    language_probs(W.d_logits.as<float>() + (size_t)s.lrow0 * V, V, e->tt.first_language_token, e->tt.num_languages,
+                   e->d_lang_probs.as<float>(), e->d_lang_arg.as<int>(), W.stream);
+    BW_CUDA(cudaMemcpyAsync(s.r->lang_out->probs, e->d_lang_probs.p, (size_t)e->tt.num_languages * 4, cudaMemcpyDeviceToHost, W.stream));
+    BW_CUDA(cudaMemcpyAsync(&s.r->lang_out->language_token, e->d_lang_arg.p, 4, cudaMemcpyDeviceToHost, W.stream));
+    BW_CUDA(cudaStreamSynchronize(W.stream));
     s.r->lang_out->n_languages = e->tt.num_languages;
   }
   for (auto& s : logit_reqs)
-    BW_CUDA(cudaMemcpyAsync(s.r->logits_out, e->grp[s.grp].d_logits.as<float>() + (size_t)s.lrow0 * V, (size_t)s.n * V * 4,
-                            cudaMemcpyDeviceToHost, e->grp[s.grp].stream));
+    BW_CUDA(cudaMemcpyAsync(s.r->logits_out, W.d_logits.as<float>() + (size_t)s.lrow0 * V, (size_t)s.n * V * 4,
+                            cudaMemcpyDeviceToHost, W.stream));
   for (auto& s : forced_reqs)  // teacher-forced test requests: the raw logits row this step sampled from
-    BW_CUDA(cudaMemcpyAsync(s.r->step_logits_out + (size_t)s.r->steps * V, e->grp[s.grp].d_logits.as<float>() + (size_t)s.lrow0 * V,
-                            (size_t)V * 4, cudaMemcpyDeviceToHost, e->grp[s.grp].stream));
-  // completion flags: one D2H behind the step on the step's own stream, one host synchronisation per step
+    BW_CUDA(cudaMemcpyAsync(s.r->step_logits_out + (size_t)s.r->steps * V, W.d_logits.as<float>() + (size_t)s.lrow0 * V,
+                            (size_t)V * 4, cudaMemcpyDeviceToHost, W.stream));
   // completion flags + the beam reorder (parent slot of every surviving hypothesis, what the page collector needs)
-  if (ng == 1) {
-    BW_CUDA(cudaMemcpyAsync(e->h_flags, e->st_step.p, e->step_out_bytes, cudaMemcpyDeviceToHost, e->grp[0].stream));
-    BW_CUDA(cudaStreamSynchronize(e->grp[0].stream));
-  } else {
-    for (int g = 0; g < ng; ++g) BW_CUDA(cudaStreamSynchronize(e->grp[g].stream));
-    BW_CUDA(cudaMemcpyAsync(e->h_flags, e->st_step.p, e->step_out_bytes, cudaMemcpyDeviceToHost, e->stream));
-    BW_CUDA(cudaStreamSynchronize(e->stream));
-  }
+  finish_step(e);
   e->stat_d2h += (long long)e->step_out_bytes;
   const unsigned char* h_src = reinterpret_cast<const unsigned char*>(e->h_flags) + (size_t)e->Q * 4;
-  e->anc_cur ^= 1;
   e->stat_steps += 1;
-  e->stat_rows += total_rows;
+  e->stat_rows += ctl.R;
 
   // bookkeeping + completion
   std::vector<Request*> still, done;
@@ -528,8 +515,6 @@ void decode_step(bw_engine* e, Ctl* ctls) {
 
 void scheduler_main(bw_engine* e) {
   cudaSetDevice(e->device);
-  Ctl ctls[kMaxGroups];
-  for (int g = 0; g < kMaxGroups; ++g) ctls[g].layout(e->grp[g].h_ctrl, e->R_max, e->LR_max, e->Q);
   const char* wenv = getenv("B200W_BATCH_WINDOW_US");
   const int window_us = wenv ? atoi(wenv) : 300;
   for (;;) {
@@ -578,7 +563,7 @@ void scheduler_main(bw_engine* e) {
     try {
       std::lock_guard<std::mutex> g(e->gpu_mu);
       if (!fresh.empty()) admit_batch(e, fresh);
-      if (!e->live.empty()) decode_step(e, ctls);
+      if (!e->live.empty()) decode_step(e);
     } catch (const std::exception& ex) {
       std::lock_guard<std::mutex> g(e->q_mu);
       fail_all(e, fresh, ex.what(), BW_ERR_CUDA);
