@@ -64,6 +64,11 @@ typedef struct bw_engine_config {
 
 #define BW_FLAG_FORCE_SIMT_GEMM 1  /* debugging: use the SIMT GEMM/attention even in bf16 mode */
 #define BW_FLAG_NO_SCHEDULER 2     /* stage-level use only (bw_mel / bw_encode / kernel tests) */
+/* bf16 compute only: keep the cached encoder K/V (cross-attention) in 8 bits -- one fp32 scale per (layer, k|v, position,
+ * head) -- for 0.53x the bytes per window and per decoder step.  Not bit-compatible with the bf16 cache: logits move
+ * by the quantisation error.  Refused (BW_ERR_INVALID) with BW_COMPUTE_FP32 or BW_FLAG_FORCE_SIMT_GEMM. */
+#define BW_FLAG_CROSS_KV_INT8 4
+#define BW_FLAG_SIMT_ATTENTION 8   /* debugging: SIMT encoder self-attention in bf16 mode */
 
 /* One tensor of the openai-whisper state dict (name = state_dict key). Host pointer. */
 typedef struct bw_tensor_desc {

@@ -102,6 +102,17 @@ int bw_test_dec_cross_attention(const void* cache, int32_t n_slots, int32_t n_la
                                 int32_t n_head, const float* q, const int32_t* grp_first, const int32_t* grp_n,
                                 const int32_t* grp_x, int32_t n_groups, int32_t max_group_rows, int32_t n_rows,
                                 int32_t force_split, void* out, void* stream);
+/* The 8-bit cross cache's quantization (BW_FLAG_CROSS_KV_INT8) on device pointers: x bf16 [n_rows][d] (d % 64 == 0) ->
+ * codes int8 [n_rows][d], scales fp32 [n_rows][d / 64]; each 64-element slice gets scale = amax / 127 and
+ * code = rint(x / scale) clamped to [-127, 127] (an all-zero slice: scale 0, codes 0). */
+int bw_test_quantize_cross_kv(const void* x, int64_t n_rows, int32_t d, int8_t* codes, float* scales, void* stream);
+/* dec_cross_attention<bf16> on the 8-bit cross cache, arguments as bw_test_dec_cross_attention: codes int8
+ * [n_slots][n_layer][T_enc][2d] (k | v) and scales fp32 [n_slots][n_layer][T_enc][2 * n_head] (k heads, then v heads),
+ * i.e. what bw_test_quantize_cross_kv makes of a bf16 cache; they are packed into the engine's slot layout first. */
+int bw_test_dec_cross_attention_int8(const int8_t* codes, const float* scales, int32_t n_slots, int32_t n_layer, int32_t layer,
+                                     int32_t T_enc, int32_t d, int32_t n_head, const float* q, const int32_t* grp_first,
+                                     const int32_t* grp_n, const int32_t* grp_x, int32_t n_groups, int32_t max_group_rows,
+                                     int32_t n_rows, int32_t force_split, void* out, void* stream);
 /* dec_self_attention<bf16> (+ fused K/V append) on device pointers over a paged pool: pages of 16 positions,
  * [n_pages][n_layer][2][16][d] bf16; page_table int32 [n_units][ceil(n_ctx / 16)]; row_page[r] = page that receives row
  * r's k / v.  max_ctx = longest context (row_pos + 1) among the rows or 0: picks the staged kernel's staging size (32 / 64 /

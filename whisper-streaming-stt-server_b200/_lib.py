@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("B200W_LIB", os.path.join(_HERE, "libb200whisper.so"))
 BW_MAX_TOKENS = 448
 BW_COMPUTE_BF16, BW_COMPUTE_FP32 = 0, 1
 BW_F32, BW_F16, BW_BF16 = 0, 1, 2
-BW_FLAG_FORCE_SIMT_GEMM, BW_FLAG_NO_SCHEDULER, BW_FLAG_SIMT_ATTENTION = 1, 2, 4
+BW_FLAG_FORCE_SIMT_GEMM, BW_FLAG_NO_SCHEDULER, BW_FLAG_CROSS_KV_INT8, BW_FLAG_SIMT_ATTENTION = 1, 2, 4, 8
 STAT_NAMES = ("kernel_launches", "decode_steps", "rows", "windows", "max_segments", "max_sequences",
               "encoder_batches", "h2d_bytes", "d2h_bytes", "kv_pages_total", "kv_pages_in_use", "kv_pages_peak", "kv_page_bytes")
 
@@ -121,6 +121,9 @@ SIGNATURES = {
     "bw_debug_trace": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_uint64), C.c_int32, c_i32_p]),
     "bw_call_decode_forced": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(DecodeOptsC), c_i32_p, C.c_int32, c_f32_p, C.POINTER(ResultC)]),
     "bw_test_dec_cross_attention": (C.c_int, [C.c_void_p] + [C.c_int32] * 6 + [C.c_void_p] * 4 + [C.c_int32] * 4 + [C.c_void_p, C.c_void_p]),
+    "bw_test_quantize_cross_kv": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bw_test_dec_cross_attention_int8": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 6 + [C.c_void_p] * 4 + [C.c_int32] * 4 +
+                                         [C.c_void_p, C.c_void_p]),
     "bw_test_dec_self_attention": (C.c_int, [C.c_int32] + [C.c_void_p] * 6 + [C.c_int32] * 3 + [C.c_void_p] * 3 +
                                    [C.c_int32] * 4 + [C.c_void_p, C.c_void_p]),
     "bw_test_self_attention_mode": (C.c_int, [C.c_int32]),

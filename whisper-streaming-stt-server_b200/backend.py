@@ -59,8 +59,10 @@ SAMPLE_RATE = 16000
 FP32_ALIASES = {"float32", "fp32"}
 BF16_ALIASES = {"bfloat16", "bf16", "default", "auto"}
 # compute types the reference's backends give another meaning to (torch_whisper.py:36-47: fp16 aliases -> .half(), int8* ->
-# float32; faster_whisper: CTranslate2 quantisation).  This engine has exactly two modes, so they run as bfloat16 -- loudly.
+# float32; faster_whisper: CTranslate2 quantisation).  This engine has no fp16 or int8-weight mode, so they run as bfloat16 -- loudly.
 REMAPPED_TO_BF16 = {"float16", "fp16", "half", "int8", "int8_float16", "int8_bfloat16", "int8_float32"}
+# bfloat16 with the cached encoder K/V (cross-attention) in 8 bits: half the decoder step's bytes, not bf16-exact
+BF16_INT8KV_ALIASES = {"bfloat16_int8kv", "bf16_int8kv"}
 _REMAP_WARNED: set = set()
 
 SUPPORTED_OPTIONS = {  # torch_whisper.py:79-97
@@ -174,6 +176,8 @@ class B200WhisperBackend:
         ct = (compute_type or "default").lower()
         if ct in FP32_ALIASES:
             self.compute = "fp32"
+        elif ct in BF16_INT8KV_ALIASES:
+            self.compute = "bf16_int8kv"
         else:
             if ct in REMAPPED_TO_BF16:
                 if ct not in _REMAP_WARNED:

@@ -83,6 +83,9 @@ int bw_engine_create(const bw_model_dims* dims, const bw_engine_config* cfg, bw_
   e->device = cfg->cuda_device;
   e->fp32 = cfg->compute == BW_COMPUTE_FP32;
   e->force_simt = (cfg->flags & BW_FLAG_FORCE_SIMT_GEMM) != 0;
+  e->cross_int8 = (cfg->flags & BW_FLAG_CROSS_KV_INT8) != 0;
+  BW_CHECK(!e->cross_int8 || (!e->fp32 && !e->force_simt),
+           "BW_FLAG_CROSS_KV_INT8 needs BW_COMPUTE_BF16 on the tensor-core path (not with BW_COMPUTE_FP32 or BW_FLAG_FORCE_SIMT_GEMM)");
   e->fuse_ln = !e->fp32 && !e->force_simt && (dims->n_text_state % 64) == 0 && getenv("B200W_NO_LN_FUSION") == nullptr;
   BW_CUDA(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
   BW_CUDA(cudaEventCreateWithFlags(&e->enc_fork, cudaEventDisableTiming));
@@ -184,7 +187,9 @@ int bw_engine_finalize(bw_engine* e) {
   engine_fold_layernorms(e);
   const size_t ts = e->fp32 ? 4 : 2;
   const size_t dm = d.n_audio_state;
-  const size_t cross_slot = (size_t)d.n_text_layer * d.n_audio_ctx * 2 * dm * ts;
+  const size_t cross_bf16 = (size_t)d.n_text_layer * d.n_audio_ctx * 2 * dm * ts;
+  const size_t cross_slot = e->cross_int8 ? (size_t)cross_int8_slot_bytes(d.n_text_layer, d.n_audio_ctx, d.n_text_head) : cross_bf16;
+  const size_t cross_stage = e->cross_int8 ? cross_bf16 : 0;
   // self-KV pool: pages of kPageTokens positions for one hypothesis slot, every layer ([L][2][kPageTokens][d]).
   // Default budget: 256 positions (16 pages) per hypothesis slot -- a decode holds at most n_initial + sample_len
   // (<= 3 + 224 without a prompt) positions per hypothesis, and beam hypotheses share the pages of their common
@@ -202,7 +207,7 @@ int bw_engine_finalize(bw_engine* e) {
   const size_t enc_per = (size_t)(3000 * 3 * d.n_mels + 3000 * dm + 1500 * 3 * dm + 1500 * dm * 2 + 1500 * 3 * dm + 1500 * dm +
                                   1500 * 4 * dm + 1500 * dm) * 4;  // upper bound (fp32 sizes)
   for (int guard = 0; guard < 64; ++guard) {
-    const double need = (double)Q * cross_slot + (double)pages_for(S) * e->page_bytes + (double)Be * enc_per;
+    const double need = (double)Q * cross_slot + (double)cross_stage + (double)pages_for(S) * e->page_bytes + (double)Be * enc_per;
     if (!(need > 0.80 * (double)free_b && (Q > 1 || S > kMaxBeam || Be > 1))) break;
     if (Q > 1) Q = std::max(1, Q * 3 / 4);
     S = std::max(kMaxBeam, std::min(S, std::max(2 * Q, kMaxBeam)));
@@ -213,6 +218,7 @@ int bw_engine_finalize(bw_engine* e) {
   e->R_max = S + 512;
   e->LR_max = S + Q + BW_MAX_TOKENS;
   e->cross_cache.alloc((size_t)Q * cross_slot);
+  if (e->cross_int8) e->cross_stage.alloc(cross_stage);
   e->n_pages = pages_for(S);
   e->self_pool.alloc((size_t)e->n_pages * e->page_bytes);
   e->d_page_table.alloc((size_t)S * e->n_blocks * 4);

@@ -18,6 +18,9 @@ namespace bw {
 void dec_cross_attention_mma(const int* group_first_row, const int* group_n_rows, const int* group_xslot, int n_groups,
                              const float* q, const CrossKV& kv, int n_layer, int layer, int d, int n_head, int n_split,
                              bf16* out, float* ws, cudaStream_t stream);
+void dec_cross_attention_int8(const int* group_first_row, const int* group_n_rows, const int* group_xslot, int n_groups,
+                              const float* q, const CrossKV& kv, int layer, int d, int n_head, int n_split, bf16* out, float* ws,
+                              cudaStream_t stream);
 
 namespace {
 
@@ -1042,11 +1045,16 @@ void dec_cross_attention(const int* group_first_row, const int* group_n_rows, co
   while (n_split < kMaxSplit && base * n_split < 4 * 148) n_split *= 2;
   if (force_split > 0) n_split = std::min(force_split, (int)kMaxSplit);  // tests: any split count, not just powers of two
   if constexpr (std::is_same<T, bf16>::value) {
-    // product mode: TMA + ldmatrix + mma.sync streaming kernel (attention_xdec.cu)
+    // product mode: TMA + ldmatrix + mma.sync streaming kernel (attention_xdec.cu), on bf16 or 8-bit K/V
     BW_CHECK(kv.n_slots > 0 && kv.n_layer > 0, "cross-attention needs the cache geometry (TMA map)");
-    dec_cross_attention_mma(group_first_row, group_n_rows, group_xslot, n_groups, q, kv, kv.n_layer, layer, d, n_head, n_split,
-                            out, workspace, stream);
+    if (kv.int8)
+      dec_cross_attention_int8(group_first_row, group_n_rows, group_xslot, n_groups, q, kv, layer, d, n_head, n_split, out,
+                               workspace, stream);
+    else
+      dec_cross_attention_mma(group_first_row, group_n_rows, group_xslot, n_groups, q, kv, kv.n_layer, layer, d, n_head, n_split,
+                              out, workspace, stream);
   } else {
+    BW_CHECK(!kv.int8, "the 8-bit cross cache needs bf16 compute");
     // fp32 validation mode: SIMT kernel with deterministic reduction order
     if (max_group_rows <= 1) launch_cross<T, 1>(group_first_row, group_n_rows, group_xslot, n_groups, q, kv, layer, d, n_head, n_split, out, workspace, stream);
     else if (max_group_rows <= 2) launch_cross<T, 2>(group_first_row, group_n_rows, group_xslot, n_groups, q, kv, layer, d, n_head, n_split, out, workspace, stream);

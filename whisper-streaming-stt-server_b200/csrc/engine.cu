@@ -3,7 +3,7 @@
 // the scheduler thread coalesces them -- the cross-session batching the reference declares
 // (config/server.yaml:48-49 decode_batch_window_ms / max_decode_batch_size) but never implements
 // (SURVEY.md section 0.4) has to live here.
-#include "engine.cuh"
+#include "sched.cuh"
 
 #include <math.h>
 #include <stdlib.h>
@@ -169,7 +169,7 @@ struct Impl {
       if constexpr (std::is_same<T, float>::value) {
         attn_encoder_simt<float>(reinterpret_cast<const float*>(qkv), reinterpret_cast<float*>(att), nb, T_enc, d.n_audio_head, st);
       } else {
-        if (e->force_simt || (e->cfg.flags & 4)) attn_encoder_simt<bf16>(reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(att), nb, T_enc, d.n_audio_head, st);
+        if (e->force_simt || (e->cfg.flags & BW_FLAG_SIMT_ATTENTION)) attn_encoder_simt<bf16>(reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(att), nb, T_enc, d.n_audio_head, st);
         else attn_encoder_tc(reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(att), nb, T_enc, d.n_audio_head, st);
       }
       {
@@ -195,16 +195,22 @@ struct Impl {
     layernorm<T>(x, e->w.ln_post_g, e->w.ln_post_b, out, M, dm, st);
   }
 
-  // cross K/V of every decoder layer for batch element `bi` -> cross-cache slot q (one launch, z = layer)
+  // cross K/V of every decoder layer for batch element `bi` -> cross-cache slot q (one launch, z = layer); the 8-bit cache
+  // takes the GEMM's bf16 output through the one-window staging buffer and quantizes it into the slot
   void cross_kv(int bi, int q) const {
     const auto& d = D();
     const int dm = d.n_text_state, T_enc = d.n_audio_ctx, L = d.n_text_layer;
     GemmArgs g;
     g.A = e->enc_out.as<T>() + (long long)bi * T_enc * dm; g.B = e->w.wkv_x; g.bias = e->w.bkv_x;
-    g.C = e->cross_cache.as<T>() + (long long)q * L * T_enc * 2 * dm;
+    g.C = e->cross_int8 ? e->cross_stage.as<T>() : e->cross_cache.as<T>() + (long long)q * L * T_enc * 2 * dm;
     g.M = T_enc; g.N = 2 * dm; g.K = dm; g.lda = dm; g.ldb = dm; g.ldc = 2 * dm;
     g.Z = L; g.a_zstride = 0; g.b_zstride = (long long)2 * dm * dm; g.c_zstride = (long long)T_enc * 2 * dm; g.bias_zstride = 2 * dm;
     gemm(g);
+    if (e->cross_int8) {
+      const CrossKV x = engine_cross_kv_desc(e);
+      cross_kv_int8_write(e->cross_stage.as<bf16>(), nullptr, nullptr, 1, L, T_enc, dm,
+                          e->cross_cache.as<unsigned char>() + (long long)q * x.slot_stride, stream);
+    }
   }
 
   // ---- one decoder step over the rows of e->dec.ctl; control block already on the device ----
@@ -238,9 +244,7 @@ struct Impl {
                  e->d_page_table.as<int>(), e->n_blocks, st);
     const SelfKV skv = self_kv();
     dec_self_pospage(rows, skv, H, st);
-    CrossKV xkv;
-    xkv.cache = e->cross_cache.p; xkv.slot_stride = (long long)L * d.n_audio_ctx * 2 * dm; xkv.T_enc = d.n_audio_ctx;
-    xkv.n_slots = e->Q; xkv.n_layer = L;
+    const CrossKV xkv = engine_cross_kv_desc(e);
     const int Ra = e->R_max;
     for (int l = 0; l < L; ++l) {
       const LayerW& w = e->w.dec[l];
@@ -288,9 +292,7 @@ struct Impl {
                        xb, lst, e->d_page_table.as<int>(), e->n_blocks, st);
     const SelfKV skv = self_kv();
     dec_self_pospage(rows, skv, H, st);
-    CrossKV xkv;
-    xkv.cache = e->cross_cache.p; xkv.slot_stride = (long long)L * d.n_audio_ctx * 2 * dm; xkv.T_enc = d.n_audio_ctx;
-    xkv.n_slots = e->Q; xkv.n_layer = L;
+    const CrossKV xkv = engine_cross_kv_desc(e);
     const int Ra = e->R_max;
     for (int l = 0; l < L; ++l) {
       const LayerW& w = e->w.dec[l];
@@ -500,6 +502,15 @@ template <typename T> static void encoder_forward_t(bw_engine* e, int nb) {
 void engine_encoder_forward(bw_engine* e, int nb) {
   if (e->fp32) encoder_forward_t<float>(e, nb); else encoder_forward_t<bf16>(e, nb);
 }
+CrossKV engine_cross_kv_desc(const bw_engine* e) {
+  const auto& d = e->dims;
+  CrossKV x;
+  x.cache = e->cross_cache.p; x.T_enc = d.n_audio_ctx; x.n_slots = e->Q; x.n_layer = d.n_text_layer; x.int8 = e->cross_int8;
+  x.slot_stride = x.int8 ? cross_int8_slot_bytes(d.n_text_layer, d.n_audio_ctx, d.n_text_head)
+                         : (long long)d.n_text_layer * d.n_audio_ctx * 2 * d.n_text_state;
+  return x;
+}
+
 void engine_cross_kv(bw_engine* e, int bi, int q) {
   if (e->fp32) Impl<float>(e).cross_kv(bi, q); else Impl<bf16>(e).cross_kv(bi, q);
 }

@@ -200,6 +200,7 @@ struct bw_engine {
   bool fp32 = false;       // validation mode
   bool force_simt = false;
   bool fuse_ln = false;    // decoder LayerNorms folded into the row GEMMs (bf16 tensor-core mode)
+  bool cross_int8 = false; // BW_FLAG_CROSS_KV_INT8: 8-bit cross cache (kernels.cuh CrossKV)
   std::vector<std::unique_ptr<bw::DevBuf>> fold_masters;                    // released by bw_engine_finalize
   std::unordered_map<std::string, float*> named_master;                     // tensor name -> fp32 master slice
   std::atomic<int> refs{1};
@@ -230,6 +231,7 @@ struct bw_engine {
   // pools
   int Q = 0, S = 0, Be = 0, R_max = 0, LR_max = 0;
   bw::DevBuf cross_cache, self_pool;
+  bw::DevBuf cross_stage;  // 8-bit mode: bf16 cross K/V of one window ([L][T_enc][2d]), quantized into its slot
   // paged self-KV: n_pages pages of kPageTokens positions ([L][2][kPageTokens][d] each), page table on the device,
   // free list + reservations on the host (scheduler thread)
   int n_pages = 0, n_blocks = 0;

@@ -137,9 +137,24 @@ void fill_random(T* p, long long n, unsigned long long seed, float scale, cudaSt
   BW_CUDA(cudaGetLastError());
 }
 void fill_cross_cache(bw_engine* e, int n_segments) {
+  if (e->cross_int8) {  // valid codes and scales: random bf16 K/V of each window through the cache's own quantizer
+    const auto& d = e->dims;
+    const CrossKV x = engine_cross_kv_desc(e);
+    for (int i = 0; i < n_segments; ++i) {
+      fill_random<bf16>(e->cross_stage.as<bf16>(), (long long)(e->cross_stage.bytes / 2), 0x5eedull + i, 1.f, e->stream);
+      cross_kv_int8_write(e->cross_stage.as<bf16>(), nullptr, nullptr, 1, d.n_text_layer, d.n_audio_ctx, d.n_text_state,
+                          e->cross_cache.as<unsigned char>() + (long long)i * x.slot_stride, e->stream);
+    }
+    return;
+  }
   const long long n = (long long)n_segments * (long long)(e->cross_cache.bytes / e->Q) / (e->fp32 ? 4 : 2);
   if (e->fp32) fill_random<float>(e->cross_cache.as<float>(), n, 0x5eedull, 1.f, e->stream);
   else fill_random<bf16>(e->cross_cache.as<bf16>(), n, 0x5eedull, 1.f, e->stream);
+}
+// algorithmic bytes of one layer's cached K/V of one window: codes + scales in the 8-bit mode
+double cross_layer_bytes(const bw_engine* e) {
+  const double d = e->dims.n_text_state, T = e->dims.n_audio_ctx;
+  return e->cross_int8 ? 2 * T * d + 2 * T * e->dims.n_text_head * 4.0 : 2 * T * d * (e->fp32 ? 4 : 2);
 }
 struct EvTimer {
   cudaEvent_t a = nullptr, b = nullptr;
@@ -271,7 +286,7 @@ int bw_bench_decoder_step(bw_engine* e, int32_t n_segments, int32_t n_group, int
   *ms_out = t.stop_ms() / iters;
   const double ts = e->fp32 ? 4 : 2, d = e->dims.n_text_state, L = e->dims.n_text_layer, V = e->dims.n_vocab;
   const double S = (double)n_segments * n_group;
-  *bytes_out = ts * (L * 14 * d * d + V * d) + n_segments * ts * L * 2 * 1500 * d + S * ts * L * 2 * (context_len + iters / 2.0) * d + 4 * S * V;
+  *bytes_out = ts * (L * 14 * d * d + V * d) + n_segments * L * cross_layer_bytes(e) + S * ts * L * 2 * (context_len + iters / 2.0) * d + 4 * S * V;
   BW_API_END
 }
 
@@ -386,8 +401,7 @@ int bw_bench_cross_attention(bw_engine* e, int32_t n_segments, int32_t n_group, 
   const int R = n_segments * n_group;
   fill_random<float>(W.d_q.as<float>(), (long long)R * dm, 0x9ull, 1.f, e->stream);
   auto run = [&](int layer) {
-    CrossKV x; x.cache = e->cross_cache.p; x.slot_stride = (long long)L * d.n_audio_ctx * 2 * dm; x.T_enc = d.n_audio_ctx;
-    x.n_slots = e->Q; x.n_layer = L;
+    const CrossKV x = engine_cross_kv_desc(e);
     if (e->fp32)
       dec_cross_attention<float>(W.dev(ctl.grp_first), W.dev(ctl.grp_n), W.dev(ctl.grp_x), n_segments, n_group, R, W.d_q.as<float>(), x,
                                  layer, dm, d.n_text_head, W.d_att.as<float>(), W.d_ws.as<float>(), e->stream);
@@ -402,7 +416,7 @@ int bw_bench_cross_attention(bw_engine* e, int32_t n_segments, int32_t n_group, 
   for (int i = 0; i < iters; ++i) run(i % L);
   *ms_out = t.stop_ms() / iters;
   const double ts = e->fp32 ? 4 : 2;
-  *bytes_out = (double)n_segments * ts * 2 * 1500 * dm + (double)R * dm * ts * 2;
+  *bytes_out = (double)n_segments * cross_layer_bytes(e) + (double)R * dm * ts * 2;
   BW_API_END
 }
 
@@ -472,6 +486,38 @@ int bw_test_dec_cross_attention(const void* cache, int32_t n_slots, int32_t n_la
   ws.alloc(dec_cross_workspace_floats(n_rows, n_head) * 4);
   CrossKV x;
   x.cache = cache; x.slot_stride = (long long)n_layer * T_enc * 2 * d; x.T_enc = T_enc; x.n_slots = n_slots; x.n_layer = n_layer;
+  dec_cross_attention<bf16>(grp_first, grp_n, grp_x, n_groups, max_group_rows, n_rows, q, x, layer, d, n_head,
+                            reinterpret_cast<bf16*>(out), ws.as<float>(), st, force_split);
+  BW_CUDA(cudaStreamSynchronize(st));
+  BW_API_END
+}
+
+int bw_test_quantize_cross_kv(const void* x, int64_t n_rows, int32_t d, int8_t* codes, float* scales, void* stream) {
+  BW_API_BEGIN
+  BW_CHECK(x && codes && scales && n_rows >= 1 && d >= 64 && d % 64 == 0, "bad argument");
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  quantize_int8_slices(reinterpret_cast<const bf16*>(x), n_rows * (d / 64), codes, scales, st);
+  BW_CUDA(cudaStreamSynchronize(st));
+  BW_API_END
+}
+
+int bw_test_dec_cross_attention_int8(const int8_t* codes, const float* scales, int32_t n_slots, int32_t n_layer, int32_t layer,
+                                     int32_t T_enc, int32_t d, int32_t n_head, const float* q, const int32_t* grp_first,
+                                     const int32_t* grp_n, const int32_t* grp_x, int32_t n_groups, int32_t max_group_rows,
+                                     int32_t n_rows, int32_t force_split, void* out, void* stream) {
+  BW_API_BEGIN
+  BW_CHECK(codes && scales && q && grp_first && grp_n && grp_x && out, "null argument");
+  BW_CHECK(n_slots >= 1 && n_layer >= 1 && layer >= 0 && layer < n_layer && d == 64 * n_head && n_groups >= 1 && n_rows >= 1 &&
+           T_enc >= 1 && T_enc <= 1504, "bad geometry");
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  CrossKV x;
+  x.slot_stride = cross_int8_slot_bytes(n_layer, T_enc, n_head); x.T_enc = T_enc; x.n_slots = n_slots; x.n_layer = n_layer;
+  x.int8 = true;
+  DevBuf cache, ws;
+  cache.alloc((size_t)(n_slots * x.slot_stride));
+  ws.alloc(dec_cross_workspace_floats(n_rows, n_head) * 4);
+  cross_kv_int8_write(nullptr, codes, scales, n_slots, n_layer, T_enc, d, cache.p, st);
+  x.cache = cache.p;
   dec_cross_attention<bf16>(grp_first, grp_n, grp_x, n_groups, max_group_rows, n_rows, q, x, layer, d, n_head,
                             reinterpret_cast<bf16*>(out), ws.as<float>(), st, force_split);
   BW_CUDA(cudaStreamSynchronize(st));

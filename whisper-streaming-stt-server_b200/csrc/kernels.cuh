@@ -118,18 +118,41 @@ void dec_self_attention(const DecRows& rows, const float* qkv, const SelfKV& kv,
 // Cross attention over the cached encoder K/V of each row's segment:
 // cross cache slot layout [L][T_enc][2*d] (k | v). Group g = rows [first_row, first_row + n_rows) that share
 // segment slot group_xslot[g] (the beams of one request); groups tile [0, n_rows) in order.
+//
+// 8-bit cross cache (BW_FLAG_CROSS_KV_INT8, bf16 mode only).  One scale per (layer, k | v, position, head):
+// scale = amax / 127 over that 64-dim head slice, code = rint(x / scale) clamped to [-127, 127]; an all-zero slice has
+// scale 0 and codes 0.  A slot is [L][n_head][ceil(T_enc / 64)] chunks of kCrossInt8ChunkBytes, one per (layer, head,
+// 64-key tile), each fetched by one bulk copy into a stage of dec_cross_attention_int8_kernel (attention_xdec.cu):
+//   [0, 4096)     K codes  [key][dim]
+//   [4096, 8192)  V codes transposed for the P.V fragments: byte w*1024 + hf*512 + (g*4 + c)*16 + i*4 + j
+//                 holds V[key w*16 + c*4 + j][dim (hf*4 + i)*8 + g]
+//   [8192, 8448)  K scales fp32 [key];  [8448, 8704)  V scales fp32 [key]
+// Keys past T_enc hold code 0, scale 0.  Only cross_kv_int8_write writes this layout and only the int8 attention
+// kernel reads it.
+constexpr int kCrossInt8ChunkBytes = 2 * 64 * 64 + 2 * 64 * 4;
+inline long long cross_int8_slot_bytes(int n_layer, int T_enc, int n_head) {
+  return (long long)n_layer * n_head * ((T_enc + 63) / 64) * kCrossInt8ChunkBytes;
+}
 struct CrossKV {
-  const void* cache = nullptr;   // T*
-  long long slot_stride = 0;     // elements per slot = L*T_enc*2*d
+  const void* cache = nullptr;   // T*, or the 8-bit chunks above
+  long long slot_stride = 0;     // elements per slot = L*T_enc*2*d; bytes per slot (cross_int8_slot_bytes) when int8
   int T_enc = 1500;
   int n_slots = 0;               // slots behind `cache` (TMA map extent)
   int n_layer = 0;
+  bool int8 = false;             // cache format: T (false) or 8-bit codes + scales
 };
 template <typename T>
 void dec_cross_attention(const int* group_first_row, const int* group_n_rows, const int* group_xslot, int n_groups,
                          int max_group_rows, int n_rows, const float* q, const CrossKV& kv, int layer, int d, int n_head, T* out,
                          float* workspace, cudaStream_t stream, int force_split = 0);
 size_t dec_cross_workspace_floats(int n_rows, int n_head);
+// Writes 8-bit slots in the layout above.  rows != nullptr: quantizes bf16 rows [n_slots][L][T_enc][2d] (k | v, the
+// cross-KV GEMM's output); else packs codes int8 [n_slots][L][T_enc][2d] + scales fp32 [n_slots][L][T_enc][2 * n_head]
+// (k heads, then v heads) that are already quantized.
+void cross_kv_int8_write(const bf16* rows, const int8_t* codes, const float* scales, int n_slots, int n_layer, int T_enc, int d,
+                         void* cache, cudaStream_t stream);
+// The same quantization on plain rows: x bf16 [n_slices][64] -> codes [n_slices][64], scales [n_slices]
+void quantize_int8_slices(const bf16* x, long long n_slices, int8_t* codes, float* scales, cudaStream_t stream);
 
 // ---- sampling.cu ----
 struct TokenTables {

@@ -17,6 +17,7 @@ void engine_build_weight_table(bw_engine* e);
 void engine_load_tensor(bw_engine* e, const bw_tensor_desc& t);
 void engine_encoder_forward(bw_engine* e, int nb);
 void engine_cross_kv(bw_engine* e, int bi, int q);
+CrossKV engine_cross_kv_desc(const bw_engine* e);  // the cross cache as the decoder step reads it
 void engine_window_to_A1(bw_engine* e, const float* logmel, int ld, int n_real, const int* gmax, int seek, int seg, int bi);
 void engine_decoder_layers(bw_engine* e);  // the step that e->dec.ctl describes, on e->dec.stream
 void engine_init_requests(bw_engine* e, const int* init_dev, int n);

@@ -124,7 +124,8 @@ class Call:
 
 
 class Engine:
-    """One weight copy + KV pools + scheduler thread on one GPU."""
+    """One weight copy + KV pools + scheduler thread on one GPU.  compute: "bf16" (product mode), "bf16_int8kv" (bf16 with the
+    cached encoder K/V in 8 bits, BW_FLAG_CROSS_KV_INT8) or "fp32" (validation mode)."""
 
     def __init__(self, dims: ModelDims, state: Dict[str, object], device_index: int = 0, compute: str = "bf16",
                  max_segments: int = 0, max_sequences: int = 0, max_encoder_batch: int = 0, flags: int = 0, max_kv_pages: int = 0):
@@ -140,6 +141,8 @@ class Engine:
         self._resampler_lock = threading.Lock()
         self._resamplers = set()
         cd = L.ModelDimsC(*[getattr(dims, f) for f, _ in L.ModelDimsC._fields_])
+        if compute == "bf16_int8kv":
+            flags |= L.BW_FLAG_CROSS_KV_INT8
         cfg = L.EngineConfigC(device_index, L.BW_COMPUTE_FP32 if compute == "fp32" else L.BW_COMPUTE_BF16, max_segments,
                               max_sequences, max_encoder_batch, flags, max_kv_pages)
         L.check(self.lib.bw_engine_create(C.byref(cd), C.byref(cfg), C.byref(self.handle)), "bw_engine_create")
