@@ -182,6 +182,25 @@ int bw_decode_many(bw_call* const* calls, const int32_t* seeks, const bw_decode_
                    int32_t* statuses, int32_t n);
 /* upstream decoding.detect_language on the window at `seek`. Blocking. */
 int bw_call_detect_language(bw_call*, int32_t seek, bw_lang_result* out);
+/* A decode that detects its own language: bw_call_decode and bw_call_detect_language of the same window in one
+ * admission, one encoder pass and one cross-KV write.  opts->initial_tokens is the sot sequence with the language left
+ * open: initial_tokens[0] = <|sot|> (sot_index 0, no prompt in front) and initial_tokens[1] = -1, the placeholder the
+ * engine fills with the detected language token, e.g. {sot, -1, transcribe [, no_timestamps]}.  The language is the
+ * arg-max over the language tokens of the <|sot|> row's logits -- the row, and the arithmetic, of
+ * bw_call_detect_language(call, seek) -- chosen on the device; `out` and `lang` then hold what bw_call_detect_language
+ * followed by bw_call_decode with that language's sot sequence return.  The detected token counts as an initial token
+ * (sample_begin, timestamp rules and log-probabilities are those of the two-call path).
+ * Detection window: the decode window at `seek`, with zeros past content_frames -- the window bw_call_detect_language
+ * uses.  (Upstream transcribe detects on the first 30 s of log-mel of the padded audio; the two coincide when
+ * content_frames - seek >= 3000.)
+ * BW_ERR_INVALID when the model has no language tokens (an English-only vocabulary, n_vocab < 51865, as upstream's
+ * is_multilingual), sot_index != 0, initial_tokens[1] != -1 or -1 appears anywhere else. */
+int bw_call_decode_detect(bw_call*, int32_t seek, const bw_decode_opts* opts, bw_result* out, bw_lang_result* lang);
+/* bw_decode_many with detect-mode windows mixed in: window i is in detect mode when its initial tokens hold the
+ * placeholder -1 (checked as above); its language goes to langs[i].  langs has one entry per window (NULL: no window is
+ * in detect mode); the entries of the other windows are zeroed. */
+int bw_decode_many_detect(bw_call* const* calls, const int32_t* seeks, const bw_decode_opts* opts, bw_result* results,
+                          bw_lang_result* langs, int32_t* statuses, int32_t n);
 int bw_call_close(bw_call*);
 
 /* ---- stage-level entry points (parity tests, ncu isolation) ---- */

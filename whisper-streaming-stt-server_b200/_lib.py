@@ -15,6 +15,7 @@ BW_MAX_TOKENS = 448
 BW_COMPUTE_BF16, BW_COMPUTE_FP32 = 0, 1
 BW_F32, BW_F16, BW_BF16 = 0, 1, 2
 BW_FLAG_FORCE_SIMT_GEMM, BW_FLAG_NO_SCHEDULER, BW_FLAG_CROSS_KV_INT8, BW_FLAG_SIMT_ATTENTION = 1, 2, 4, 8
+LANGUAGE_PLACEHOLDER = -1  # initial_tokens[1] of a detect-mode decode (bw_call_decode_detect): the engine fills it
 STAT_NAMES = ("kernel_launches", "decode_steps", "rows", "windows", "max_segments", "max_sequences",
               "encoder_batches", "h2d_bytes", "d2h_bytes", "kv_pages_total", "kv_pages_in_use", "kv_pages_peak", "kv_page_bytes")
 
@@ -100,6 +101,9 @@ SIGNATURES = {
     "bw_call_decode": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(DecodeOptsC), C.POINTER(ResultC)]),
     "bw_decode_many": (C.c_int, [C.POINTER(C.c_void_p), c_i32_p, C.POINTER(DecodeOptsC), C.POINTER(ResultC), c_i32_p, C.c_int32]),
     "bw_call_detect_language": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(LangResultC)]),
+    "bw_call_decode_detect": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(DecodeOptsC), C.POINTER(ResultC), C.POINTER(LangResultC)]),
+    "bw_decode_many_detect": (C.c_int, [C.POINTER(C.c_void_p), c_i32_p, C.POINTER(DecodeOptsC), C.POINTER(ResultC),
+                                        C.POINTER(LangResultC), c_i32_p, C.c_int32]),
     "bw_call_close": (C.c_int, [C.c_void_p]),
     "bw_mel": (C.c_int, [C.c_void_p, c_f32_p, C.c_int64, C.c_int32, c_f32_p, c_i32_p]),
     "bw_encode": (C.c_int, [C.c_void_p, c_f32_p, C.c_int32, c_f32_p]),

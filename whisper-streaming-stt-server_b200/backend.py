@@ -31,6 +31,7 @@ from typing import Any, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
+from ._lib import LANGUAGE_PLACEHOLDER
 from .engine import Engine
 from .synth import MODEL_DIMS, LazyRandomState, ModelDims, random_state_dict
 from .vocab import Detokenizer, Vocab, normalize_language, vocab_for
@@ -200,6 +201,9 @@ class B200WhisperBackend:
         self.honor_without_timestamps = os.environ.get("B200_WHISPER_HONOR_WITHOUT_TIMESTAMPS", "0") == "1"
         self.report_language_probability = os.environ.get("B200_WHISPER_REPORT_LANGUAGE_PROB", "0") == "1"
         self.last_language_probability: Optional[float] = None
+        # language unset: detect it inside the first window's decode (one encoder pass) where the engine can; False runs
+        # upstream's separate detect_language pass first, as engines without that capability do
+        self.detect_in_decode = bool(getattr(self.engine, "detects_in_decode", False))
         env_seed = os.environ.get("B200_WHISPER_SEED")
         self.base_seed = int(env_seed) & _M64 if env_seed else int.from_bytes(os.urandom(8), "little")
         self._call_counter = itertools.count()
@@ -322,7 +326,9 @@ class B200WhisperBackend:
         try:
             call, seek, kw = next(gen)
             while True:
-                call, seek, kw = gen.send(call.decode(seek, **kw))
+                kw = dict(kw)
+                res = call.decode_detect(seek, **kw) if kw.pop("detect", False) else call.decode(seek, **kw)
+                call, seek, kw = gen.send(res)
         except StopIteration as stop:
             return stop.value
 
@@ -364,18 +370,28 @@ class B200WhisperBackend:
         with self.engine.open_call(audio, sample_rate) as call:
             content_frames = call.content_frames
             language_probability = None
+            # Language unset on a multilingual model: upstream detects it once per call on the window at seek 0.  When
+            # nothing precedes that window's <|sot|> (no initial_prompt), its first decode attempt detects the language
+            # itself (Call.decode_detect: one encoder pass for both); otherwise -- or with detect_in_decode off -- a
+            # separate detect_language pass runs first.
+            detect_first = False
             if language is None:
                 if not v.multilingual:
                     language = "en"
+                elif initial_prompt is None and content_frames > 0 and self.detect_in_decode:
+                    detect_first = True
                 else:
                     tok, probs = call.detect_language(0)
                     language = v.language_of_token(tok)
                     language_probability = float(probs[tok - v.first_language_token])
             else:
                 language = normalize_language(language)
-            sot_sequence = v.sot_sequence(language, task)
-            if without_ts:
-                sot_sequence = sot_sequence + [v.no_timestamps]
+
+            def sot_sequence_of(lang: Optional[str]) -> List[int]:
+                seq = v.sot_sequence(lang, task)
+                return seq + [v.no_timestamps] if without_ts else seq
+
+            sot_sequence = sot_sequence_of(language)
             n_ctx = self.engine.dims.n_text_ctx
 
             all_tokens: List[int] = []
@@ -408,7 +424,16 @@ class B200WhisperBackend:
                               length_penalty=length_penalty, sample_len=int(sample_len or 0), without_timestamps=without_ts)
                     if t > 0:
                         kw.update(beam_size=None, patience=None, temperature=t, best_of=n_best, seed=window_seed(call_seed, seek, attempt))
+                    if detect_first:  # the first window has no prompt: initial == sot_sequence, sot at index 0
+                        kw.update(initial=[v.sot, LANGUAGE_PLACEHOLDER] + initial[2:], detect=True)
                     res = dict((yield call, seek, kw))
+                    if detect_first:  # later rungs and windows decode with the detected language, as upstream's
+                        detect_first = False
+                        tok = res.pop("language_token")
+                        language = v.language_of_token(tok)
+                        language_probability = float(res.pop("language_probs")[tok - v.first_language_token])
+                        sot_sequence = sot_sequence_of(language)
+                        initial = list(sot_sequence)
                     res["temperature"] = t
                     text_all = self.detok.decode([tk for tk in res["tokens"] if tk < v.eot]).strip()
                     res["compression_ratio"] = compression_ratio(text_all)

@@ -257,6 +257,9 @@ int bw_engine_finalize(bw_engine* e) {
   // rows past the live count are read (and discarded) by the GEMMs' TMA boxes: keep them finite
   for (DevBuf* b : {&W.d_xn, &W.d_qkv, &W.d_att, &W.d_q, &W.d_h, &W.d_lnrows}) BW_CUDA(cudaMemset(b->p, 0, b->bytes));
   e->d_lang_probs.alloc(128 * 4); e->d_lang_arg.alloc(4);
+  e->d_det_probs.alloc((size_t)Q * kMaxLanguages * 4); e->d_det_tok.alloc((size_t)Q * 4);
+  BW_CUDA(cudaMemset(e->d_det_probs.p, 0, e->d_det_probs.bytes));
+  BW_CUDA(cudaMemset(e->d_det_tok.p, 0, e->d_det_tok.bytes));
   BW_CUDA(cudaMemset(e->self_pool.p, 0, e->self_pool.bytes));
   // decoder state
   const size_t n_ctx = d.n_text_ctx;
@@ -531,8 +534,23 @@ int bw_call_decode(bw_call* c, int32_t seek, const bw_decode_opts* o, bw_result*
   BW_API_END
 }
 
+int bw_call_decode_detect(bw_call* c, int32_t seek, const bw_decode_opts* o, bw_result* out, bw_lang_result* lang) {
+  BW_API_BEGIN
+  BW_CHECK(lang, "null argument");
+  Request r;
+  fill_decode_request(r, c, seek, o, out, lang);
+  const int st = submit_and_wait(c->eng, r);
+  if (st != BW_OK) return st;
+  BW_API_END
+}
+
 int bw_decode_many(bw_call* const* calls, const int32_t* seeks, const bw_decode_opts* opts, bw_result* results,
                    int32_t* statuses, int32_t n) {
+  return bw_decode_many_detect(calls, seeks, opts, results, nullptr, statuses, n);
+}
+
+int bw_decode_many_detect(bw_call* const* calls, const int32_t* seeks, const bw_decode_opts* opts, bw_result* results,
+                          bw_lang_result* langs, int32_t* statuses, int32_t n) {
   BW_API_BEGIN
   BW_CHECK(calls && seeks && opts && results && n >= 0, "null argument");
   std::vector<std::unique_ptr<Request>> reqs;
@@ -540,8 +558,13 @@ int bw_decode_many(bw_call* const* calls, const int32_t* seeks, const bw_decode_
   bw_engine* e = n > 0 && calls[0] ? calls[0]->eng : nullptr;
   for (int i = 0; i < n; ++i) {
     BW_CHECK(calls[i] && calls[i]->eng == e, "all calls of a batch must belong to one engine");
+    // detect mode: the window's initial tokens hold the language placeholder (fill_decode_request checks where)
+    const bw_decode_opts& o = opts[i];
+    const bool detect = langs && o.initial_tokens && o.n_initial > 0 &&
+                        std::find(o.initial_tokens, o.initial_tokens + o.n_initial, kLanguagePlaceholder) != o.initial_tokens + o.n_initial;
+    if (langs && !detect) memset(&langs[i], 0, sizeof(langs[i]));
     reqs.emplace_back(new Request());
-    fill_decode_request(*reqs.back(), calls[i], seeks[i], &opts[i], &results[i]);
+    fill_decode_request(*reqs.back(), calls[i], seeks[i], &o, &results[i], detect ? &langs[i] : nullptr);
     ptrs.push_back(reqs.back().get());
   }
   if (n == 0) return BW_OK;

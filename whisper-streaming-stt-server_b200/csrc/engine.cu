@@ -15,7 +15,7 @@ namespace bw {
 
 namespace {
 
-__global__ void init_requests_kernel(const int* __restrict__ init, int n, ReqState rs, SeqState ss, int anc_cur, int n_ctx) {
+__global__ void init_requests_kernel(const int* __restrict__ init, int n, ReqState rs, SeqState ss, int n_ctx) {
   // init record: q, G, greedy, sample_begin, cur_len, first_seq, without_ts, suppress_blank, max_initial_ts,
   //              max_candidates, last_init_tok, temperature (float bits), seed_lo, seed_hi, pad, pad
   const int* r = init + blockIdx.x * kInitRecInts;
@@ -32,13 +32,18 @@ __global__ void init_requests_kernel(const int* __restrict__ init, int n, ReqSta
       ss.seq_first[s] = first_seq | (G == 1 ? 0x40000000 : 0);  // kSingleBeamFlag: ancestry is identically 0
     }
   }
-  unsigned char* a = ss.anc[anc_cur] + (long long)first_seq * n_ctx;
-  for (int i = threadIdx.x; i < G * n_ctx; i += blockDim.x) a[i] = 0;
+  // Both ancestry buffers: the one current at the request's first sampling step is anc_cur for a decode prefilled in its
+  // admission step, the other one for a detect-mode decode (its sot step flips anc_cur before any beam update), and the
+  // sequence slots still hold the previous occupant's ancestry.
+  unsigned char* a0 = ss.anc[0] + (long long)first_seq * n_ctx;
+  unsigned char* a1 = ss.anc[1] + (long long)first_seq * n_ctx;
+  for (int i = threadIdx.x; i < G * n_ctx; i += blockDim.x) { a0[i] = 0; a1[i] = 0; }
 }
 
-// Finished requests -> one contiguous blob each (layout: finalize_decode in api.cu), so that the host needs ONE
+// Finished requests -> one contiguous blob each (layout: finalize_decode in scheduler.cu), so that the host needs ONE
 // device-to-host copy per step instead of eight per finished request.
 __global__ void gather_final_kernel(const int* __restrict__ list, ReqState rs, SeqState ss, int n_ctx, int blob_bytes,
+                                    const int* __restrict__ det_tok, const float* __restrict__ det_probs,
                                     unsigned char* __restrict__ out) {
   const int q = list[blockIdx.x * 3], first_seq = list[blockIdx.x * 3 + 1], G = list[blockIdx.x * 3 + 2];
   unsigned char* b = out + (size_t)blockIdx.x * blob_bytes;
@@ -60,6 +65,10 @@ __global__ void gather_final_kernel(const int* __restrict__ list, ReqState rs, S
   unsigned char* par = reinterpret_cast<unsigned char*>(tok + (size_t)n_ctx * kMaxBeam);
   const unsigned char* psrc = rs.parent + (size_t)q * n_ctx * kMaxBeam;
   for (int i = threadIdx.x; i < n_ctx * kMaxBeam; i += blockDim.x) par[i] = psrc[i];
+  // the language slot (meaningful for detect-mode decodes only): token, then kMaxLanguages probabilities
+  int* lang = reinterpret_cast<int*>(par + (size_t)n_ctx * kMaxBeam);
+  if (threadIdx.x == 0) lang[0] = det_tok[q];
+  for (int i = threadIdx.x; i < kMaxLanguages; i += blockDim.x) reinterpret_cast<float*>(lang)[1 + i] = det_probs[q * kMaxLanguages + i];
 }
 
 inline float bf16_bits_to_float(uint16_t b) {
@@ -523,13 +532,14 @@ void engine_decoder_layers(bw_engine* e) {
 }
 void engine_gather_final(bw_engine* e, const int* list_dev, int n, int blob_bytes, unsigned char* out_dev) {
   if (n <= 0) return;
-  gather_final_kernel<<<n, 256, 0, e->stream>>>(list_dev, e->rs, e->ss, e->dims.n_text_ctx, blob_bytes, out_dev);
+  gather_final_kernel<<<n, 256, 0, e->stream>>>(list_dev, e->rs, e->ss, e->dims.n_text_ctx, blob_bytes, e->d_det_tok.as<int>(),
+                                                e->d_det_probs.as<float>(), out_dev);
   BW_CUDA(cudaGetLastError());
   ++g_kernel_launches;
 }
 void engine_init_requests(bw_engine* e, const int* init_dev, int n) {
   if (n <= 0) return;
-  init_requests_kernel<<<n, 128, 0, e->stream>>>(init_dev, n, e->rs, e->ss, e->anc_cur, e->dims.n_text_ctx);
+  init_requests_kernel<<<n, 128, 0, e->stream>>>(init_dev, n, e->rs, e->ss, e->dims.n_text_ctx);
   BW_CUDA(cudaGetLastError());
   ++g_kernel_launches;
 }

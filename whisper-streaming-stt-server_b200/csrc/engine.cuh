@@ -72,16 +72,16 @@ struct ModelW {
 enum ReqKind { REQ_DECODE = 0, REQ_LANG = 1, REQ_LOGITS = 2 };
 
 struct StepGraphKey {
-  int R, NG, LR, SR, NA, NNS, max_grp, anc, self_chunk;  // self_chunk: the self-attention launch geometry (dec_self_chunk)
+  int R, NG, LR, SR, NA, NNS, ND, max_grp, anc, self_chunk;  // self_chunk: the self-attention launch geometry (dec_self_chunk)
   bool operator==(const StepGraphKey& o) const {
-    return R == o.R && NG == o.NG && LR == o.LR && SR == o.SR && NA == o.NA && NNS == o.NNS && max_grp == o.max_grp && anc == o.anc &&
-           self_chunk == o.self_chunk;
+    return R == o.R && NG == o.NG && LR == o.LR && SR == o.SR && NA == o.NA && NNS == o.NNS && ND == o.ND && max_grp == o.max_grp &&
+           anc == o.anc && self_chunk == o.self_chunk;
   }
 };
 struct StepGraphKeyHash {
   size_t operator()(const StepGraphKey& k) const {
     size_t h = 1469598103934665603ull;
-    for (int v : {k.R, k.NG, k.LR, k.SR, k.NA, k.NNS, k.max_grp, k.anc, k.self_chunk}) h = (h ^ (size_t)v) * 1099511628211ull;
+    for (int v : {k.R, k.NG, k.LR, k.SR, k.NA, k.NNS, k.ND, k.max_grp, k.anc, k.self_chunk}) h = (h ^ (size_t)v) * 1099511628211ull;
     return h;
   }
 };
@@ -96,10 +96,11 @@ constexpr size_t kMaxStepGraphs = 128;  // per engine; least recently used half 
 struct Ctl {
   int *row_seq, *row_pos, *row_tok, *row_bpos, *row_page, *grp_first, *grp_n, *grp_x, *lrow_src, *srow_lrow, *srow_req, *srow_seq, *act_req,
       *act_first, *act_force, *ns_lrow, *ns_req;
+  int *det_lrow, *det_req;  // detect-mode decodes whose <|sot|> row this step feeds (detect_language)
   int* base = nullptr;
   size_t total = 0;
   // fill counters of the step being built
-  int R = 0, NG = 0, LR = 0, SR = 0, NA = 0, NNS = 0, max_grp = 1, max_ctx = 0;
+  int R = 0, NG = 0, LR = 0, SR = 0, NA = 0, NNS = 0, ND = 0, max_grp = 1, max_ctx = 0;
   void layout(int* b, int Rm, int LRm, int Q) {
     base = b;
     int* p = b;
@@ -108,9 +109,10 @@ struct Ctl {
     grp_first = take(Rm); grp_n = take(Rm); grp_x = take(Rm);
     lrow_src = take(LRm); srow_lrow = take(LRm); srow_req = take(LRm); srow_seq = take(LRm);
     act_req = take(Q); act_first = take(Q); act_force = take(Q); ns_lrow = take(Q); ns_req = take(Q);
+    det_lrow = take(Q); det_req = take(Q);
     total = (size_t)(p - b);
   }
-  void reset() { R = NG = LR = SR = NA = NNS = 0; max_grp = 1; max_ctx = 0; }
+  void reset() { R = NG = LR = SR = NA = NNS = ND = 0; max_grp = 1; max_ctx = 0; }
 };
 
 // Decoder-step working set: activations, logits, control block and step graphs, with the step's own stream.
@@ -184,8 +186,13 @@ struct Request {
   std::vector<int> pages;
   std::vector<unsigned char> ref_mask;
   int pages_reserved = 0, n_blocks_max = 0;
+  // detect mode (bw_call_decode_detect): initial[1] is the language placeholder (-1); the decode is prefilled in two
+  // steps, <|sot|> alone (its logits row picks the language on the device), then positions [1, n_initial) -- see
+  // decode_step.  The language comes back through lang_out.
+  bool detect = false;
   // runtime
   int q = -1, first_seq = -1, G = 1, cur_len = 0, steps = 0;
+  int prefill_pos = 0;  // first initial position the next prefill step feeds (1 after a detect-mode decode's first step)
   bool prefilled = false;
   int batch_index = -1;  // position inside the current encoder batch
   Clock::time_point t_submit, t_admit, t_encoded;
@@ -245,6 +252,7 @@ struct bw_engine {
   // decoder activations
   bw::DecWorkspace dec;
   bw::DevBuf d_lang_probs, d_lang_arg;
+  bw::DevBuf d_det_probs, d_det_tok;  // detect-mode decodes: [Q][kMaxLanguages] probabilities, [Q] language token
   // decoder state
   bw::DevBuf st_int, st_float, st_anc0, st_anc1, st_tok, st_parent, st_step;  // st_step: [Q] completed | [Q][kMaxBeam] last_src
   bw::ReqState rs{};

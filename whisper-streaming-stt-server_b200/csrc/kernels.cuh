@@ -216,5 +216,10 @@ void no_speech_prob(const float* logits, int ld, int V, const int* lrows, const 
 // detect_language: softmax over the language tokens of one logits row
 void language_probs(const float* logits, int V, int first_lang, int n_lang, float* probs_out, int* argmax_out,
                     cudaStream_t stream);
+// The same for the n detect-mode decodes of a step at once: request reqs[i] reads logits row lrows[i]; its language
+// token goes to lang_tok[q] and next_tok[first_seq[q]], its probabilities to probs[q][0, num_languages)
+constexpr int kMaxLanguages = 128;
+void detect_language(const float* logits, int ld, const int* lrows, const int* reqs, int n, const TokenTables& tt, const ReqState& rs,
+                     const SeqState& ss, float* probs, int* lang_tok, cudaStream_t stream);
 
 }  // namespace bw

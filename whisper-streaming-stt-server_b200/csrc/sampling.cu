@@ -381,9 +381,11 @@ no_speech_kernel(const float* __restrict__ logits, int ld, int V, const int* __r
   if (threadIdx.x == 0) out_prob[reqs[blockIdx.x]] = expf(x[no_speech_id] - m) / s;
 }
 
-__global__ void __launch_bounds__(128)
-language_probs_kernel(const float* __restrict__ logits, int first_lang, int n_lang, float* __restrict__ probs,
-                      int* __restrict__ argmax_out) {
+// upstream detect_language on one logits row, for a block of 128 threads: every logit but the language tokens'
+// masked, arg-max (lowest id on ties) and softmax.  probs[i] = P(first_lang + i); returns the arg-max token id in every
+// thread.  Both detection paths (language_probs_kernel, detect_language_kernel) run exactly this arithmetic.
+__device__ __forceinline__ int language_softmax_argmax(const float* __restrict__ logits, int first_lang, int n_lang,
+                                                       float* __restrict__ probs) {
   __shared__ float sv[128];
   __shared__ int si[128];
   const int t = threadIdx.x;
@@ -405,7 +407,30 @@ language_probs_kernel(const float* __restrict__ logits, int first_lang, int n_la
     __syncthreads();
   }
   if (t < n_lang) probs[t] = e / sv[0];
-  if (t == 0) *argmax_out = first_lang + am;
+  return first_lang + am;
+}
+
+__global__ void __launch_bounds__(128)
+language_probs_kernel(const float* __restrict__ logits, int first_lang, int n_lang, float* __restrict__ probs,
+                      int* __restrict__ argmax_out) {
+  const int tok = language_softmax_argmax(logits, first_lang, n_lang, probs);
+  if (threadIdx.x == 0) *argmax_out = tok;
+}
+
+// One block per detect-mode decode in the step that fed its <|sot|> row: the language token goes to the request's
+// language slot and to next_tok of its first hypothesis, which the next step's language row embeds (row_tok = -1).
+__global__ void __launch_bounds__(128)
+detect_language_kernel(const float* __restrict__ logits, int ld, const int* __restrict__ lrows, const int* __restrict__ reqs,
+                       int first_lang, int n_lang, const ReqState rs, const SeqState ss, float* __restrict__ probs,
+                       int* __restrict__ lang_tok) {
+  pdl_trigger();
+  pdl_wait();
+  const int q = reqs[blockIdx.x];
+  const int tok = language_softmax_argmax(logits + (long long)lrows[blockIdx.x] * ld, first_lang, n_lang, probs + (long long)q * kMaxLanguages);
+  if (threadIdx.x == 0) {
+    lang_tok[q] = tok;
+    ss.next_tok[rs.first_seq[q]] = tok;
+  }
 }
 
 }  // namespace
@@ -441,6 +466,15 @@ void language_probs(const float* logits, int V, int first_lang, int n_lang, floa
   BW_CHECK(n_lang <= 128, "too many languages");
   language_probs_kernel<<<1, 128, 0, stream>>>(logits, first_lang, n_lang, probs_out, argmax_out);
   BW_CUDA(cudaGetLastError());
+  ++g_kernel_launches;
+}
+
+void detect_language(const float* logits, int ld, const int* lrows, const int* reqs, int n, const TokenTables& tt, const ReqState& rs,
+                     const SeqState& ss, float* probs, int* lang_tok, cudaStream_t stream) {
+  if (n <= 0) return;
+  BW_CHECK(tt.num_languages > 0 && tt.num_languages <= kMaxLanguages, "language detection needs 1 to 128 language tokens");
+  launch_kernel(detect_language_kernel, dim3(n), dim3(128), 0, stream, logits, ld, lrows, reqs, tt.first_language_token, tt.num_languages,
+                rs, ss, probs, lang_tok);
   ++g_kernel_launches;
 }
 

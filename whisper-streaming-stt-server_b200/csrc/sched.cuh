@@ -49,8 +49,10 @@ int page_collector_replay(int G, int n_init, int n_steps, const unsigned char* p
 int submit_and_wait(bw_engine* e, Request& r);
 // one host thread hands a whole batch to the scheduler and waits for every request of it
 int submit_many_and_wait(bw_engine* e, const std::vector<Request*>& rs);
-// validates `opts` and fills the decode fields of `r` (shared by bw_call_decode, bw_decode_many and the test hooks)
-void fill_decode_request(Request& r, bw_call* c, int seek, const bw_decode_opts* o, bw_result* out);
+// validates `opts` and fills the decode fields of `r` (shared by bw_call_decode, bw_decode_many and the test hooks).
+// lang != nullptr: detect mode (bw_call_decode_detect), initial_tokens[1] holds kLanguagePlaceholder.
+constexpr int kLanguagePlaceholder = -1;
+void fill_decode_request(Request& r, bw_call* c, int seek, const bw_decode_opts* o, bw_result* out, bw_lang_result* lang = nullptr);
 size_t fin_blob_bytes(bw_engine* e);
 // one finished request's blob (engine_gather_final) -> r->out: the ranker's pick among the request's hypotheses
 void finalize_decode(bw_engine* e, Request* r, const unsigned char* blob);

@@ -30,6 +30,8 @@ void enqueue_step_eager(bw_engine* e) {
   static const bool use_pdl = getenv("B200W_NO_PDL") == nullptr;
   PdlScope pdl(use_pdl && !e->fp32);
   no_speech_prob(logits, V, V, W.dev(c.ns_lrow), W.dev(c.ns_req), c.NNS, e->tt.no_speech, e->rs.no_speech_prob, W.stream);
+  detect_language(logits, V, W.dev(c.det_lrow), W.dev(c.det_req), c.ND, e->tt, e->rs, e->ss, e->d_det_probs.as<float>(),
+                  e->d_det_tok.as<int>(), W.stream);
   sample_topk(logits, V, V, W.dev(c.srow_lrow), W.dev(c.srow_req), W.dev(c.srow_seq), c.SR, e->tt, e->rs, e->ss, e->anc_cur,
               W.d_cand_tok.as<int>(), W.d_cand_lp.as<float>(), W.stream);
   beam_update(W.dev(c.act_req), W.dev(c.act_first), W.dev(c.act_force), c.NA, e->tt, e->rs, e->ss, e->anc_cur, e->dims.n_text_ctx,
@@ -46,7 +48,7 @@ void enqueue_step(bw_engine* e) {
   e->stat_h2d += (long long)c.total * 4;
   static const bool use_graphs = getenv("B200W_NO_GRAPH") == nullptr;
   if (!use_graphs) return enqueue_step_eager(e);
-  const StepGraphKey key{c.R, c.NG, c.LR, c.SR, c.NA, c.NNS, c.max_grp, e->anc_cur, dec_self_chunk(c.max_ctx)};
+  const StepGraphKey key{c.R, c.NG, c.LR, c.SR, c.NA, c.NNS, c.ND, c.max_grp, e->anc_cur, dec_self_chunk(c.max_ctx)};
   StepGraph& sg = W.graphs[key];
   sg.last_use = ++W.graph_clock;
   if (sg.exec) {
@@ -294,11 +296,18 @@ void finalize_decode(bw_engine* e, Request* r, const unsigned char* blob) {
   o->avg_logprob = (float)((double)cand_lp[best] / (double)(sel.size() + 1));
   o->no_speech_prob = fmisc[0];
   o->n_steps = r->steps;
+  if (r->detect) {  // the language slot behind the parents: token, then the probabilities
+    const int* lang = reinterpret_cast<const int*>(parent + (size_t)n_ctx * kMaxBeam);
+    bw_lang_result* l = r->lang_out;
+    l->language_token = lang[0];
+    l->n_languages = e->tt.num_languages;
+    memcpy(l->probs, lang + 1, (size_t)e->tt.num_languages * 4);
+  }
 }
 
 size_t fin_blob_bytes(bw_engine* e) {
   return (size_t)kMaxFinished * 12 + 4 + 4 + kMaxBeam * 4 + (size_t)e->dims.n_text_ctx * kMaxBeam * 4 +
-         (size_t)e->dims.n_text_ctx * kMaxBeam + 64;
+         (size_t)e->dims.n_text_ctx * kMaxBeam + 4 + kMaxLanguages * 4 + 64;
 }
 
 namespace {
@@ -375,22 +384,32 @@ void decode_step(bw_engine* e) {
     int &R = ctl.R, &NG = ctl.NG, &LR = ctl.LR, &SR = ctl.SR, &NA = ctl.NA, &NNS = ctl.NNS, &max_grp = ctl.max_grp;
     if (!r->prefilled) {
       const int n_init = (int)r->initial.size();
+      // Initial positions [t0, t1) are fed in this step.  A detect-mode decode takes two steps: first <|sot|> alone,
+      // whose logits row detect_language reads, then [1, n_init) -- its language row (row_tok -1) embeds the
+      // next_tok that detect_language wrote, and its sot K/V come from the page like any cached position.
+      const bool detect_sot = r->detect && r->prefill_pos == 0;
+      const int t0 = r->prefill_pos, t1 = detect_sot ? 1 : n_init;
       const int row0 = R;
-      ctl.max_ctx = std::max(ctl.max_ctx, n_init);
-      for (int t = 0; t < n_init; ++t) {
-        ctl.row_seq[R] = r->first_seq; ctl.row_pos[R] = t; ctl.row_tok[R] = r->initial[t]; ctl.row_bpos[R] = 0;
+      ctl.max_ctx = std::max(ctl.max_ctx, t1);
+      for (int t = t0; t < t1; ++t) {
+        ctl.row_seq[R] = r->first_seq; ctl.row_pos[R] = t; ctl.row_tok[R] = r->initial[t]; ctl.row_bpos[R] = t0;
         ctl.row_page[R] = kv_page_of(e, r, 0, t / kPageTokens);
         ++R;
       }
       // every hypothesis starts as a copy of slot 0's prefix
       for (int j = 0; j < r->G; ++j)
-        for (int b = 0; b <= (n_init - 1) / kPageTokens; ++b) r->ref_mask[(size_t)j * e->n_blocks + b] |= 1u;
-      for (int t = 0; t < n_init; t += 8) {
-        ctl.grp_first[NG] = row0 + t; ctl.grp_n[NG] = std::min(8, n_init - t); ctl.grp_x[NG] = r->q;
+        for (int b = 0; b <= (t1 - 1) / kPageTokens; ++b) r->ref_mask[(size_t)j * e->n_blocks + b] |= 1u;
+      for (int t = t0; t < t1; t += 8) {
+        ctl.grp_first[NG] = row0 + t - t0; ctl.grp_n[NG] = std::min(8, t1 - t); ctl.grp_x[NG] = r->q;
         max_grp = std::max(max_grp, ctl.grp_n[NG]);
         ++NG;
       }
-      if (r->kind == REQ_LANG) {
+      if (detect_sot) {  // the sot row: no_speech_prob and the language, nothing sampled yet
+        ctl.lrow_src[LR] = row0;
+        ctl.ns_lrow[NNS] = LR; ctl.ns_req[NNS] = r->q; ++NNS;
+        ctl.det_lrow[ctl.ND] = LR; ctl.det_req[ctl.ND] = r->q; ++ctl.ND;
+        ++LR;
+      } else if (r->kind == REQ_LANG) {
         ctl.lrow_src[LR] = row0;
         lang_reqs.push_back({r, LR, 1});
         ++LR;
@@ -398,14 +417,16 @@ void decode_step(bw_engine* e) {
         logit_reqs.push_back({r, LR, n_init});
         for (int t = 0; t < n_init; ++t) ctl.lrow_src[LR++] = row0 + t;
       } else {
-        const int last_row = row0 + n_init - 1;
-        int sot_lrow;
-        if (r->sot_index != n_init - 1) {
-          ctl.lrow_src[LR] = row0 + r->sot_index;
-          sot_lrow = LR++;
-        } else sot_lrow = LR;
+        const int last_row = R - 1;
+        if (!r->detect) {  // (a detect-mode decode took no_speech_prob from its sot step)
+          int sot_lrow;
+          if (r->sot_index != n_init - 1) {
+            ctl.lrow_src[LR] = row0 + r->sot_index;
+            sot_lrow = LR++;
+          } else sot_lrow = LR;
+          ctl.ns_lrow[NNS] = sot_lrow; ctl.ns_req[NNS] = r->q; ++NNS;
+        }
         ctl.lrow_src[LR] = last_row;
-        ctl.ns_lrow[NNS] = sot_lrow; ctl.ns_req[NNS] = r->q; ++NNS;
         ctl.act_req[NA] = r->q; ctl.act_first[NA] = SR; ctl.act_force[NA] = forced_token(r); ++NA;
         ctl.srow_lrow[SR] = LR; ctl.srow_req[SR] = r->q; ctl.srow_seq[SR] = r->first_seq; ++SR;
         if (r->step_logits_out) forced_reqs.push_back({r, LR, 1});
@@ -455,6 +476,11 @@ void decode_step(bw_engine* e) {
   std::vector<Request*> still, done;
   for (Request* r : e->live) {
     if (r->kind != REQ_DECODE) { done.push_back(r); continue; }
+    if (r->detect && r->prefill_pos == 0) {  // its sot step: the language is chosen, nothing was sampled
+      r->prefill_pos = 1;
+      still.push_back(r);
+      continue;
+    }
     r->prefilled = true;
     r->cur_len += 1;
     r->steps += 1;
@@ -534,7 +560,11 @@ void scheduler_main(bw_engine* e) {
         e->q_cv.wait_for(lk, std::chrono::microseconds(window_us), [&] { return e->stop || (int)e->pending.size() >= e->Be; });
       }
       int rows = 0, lrows = 0;
-      for (Request* r : e->live) { rows += r->G; lrows += r->G; }
+      // rows / logits rows of the live requests in the next step (a detect-mode decode past its sot step still prefills)
+      for (Request* r : e->live) {
+        rows += r->prefilled ? r->G : (int)r->initial.size() - r->prefill_pos;
+        lrows += r->prefilled ? r->G : 2;
+      }
       while (!e->pending.empty() && (int)fresh.size() < e->Be) {
         Request* r = e->pending.front();
         const int n_init = (int)r->initial.size();
@@ -587,7 +617,7 @@ int submit_many_and_wait(bw_engine* e, const std::vector<Request*>& rs) {
   return BW_OK;
 }
 
-void fill_decode_request(Request& r, bw_call* c, int seek, const bw_decode_opts* o, bw_result* out) {
+void fill_decode_request(Request& r, bw_call* c, int seek, const bw_decode_opts* o, bw_result* out, bw_lang_result* lang) {
   BW_CHECK(c && o && out, "null argument");
   bw_engine* e = c->eng;
   BW_CHECK(o->n_initial >= 1 && o->initial_tokens, "initial tokens required");
@@ -596,7 +626,26 @@ void fill_decode_request(Request& r, bw_call* c, int seek, const bw_decode_opts*
   BW_CHECK(o->sot_index >= 0 && o->sot_index < o->n_initial, "sot_index out of range");
   BW_CHECK(o->beam_size >= 0 && o->beam_size <= kMaxBeam, "beam_size must be in [0, 8]");
   BW_CHECK(seek >= 0, "negative seek");
-  for (int i = 0; i < o->n_initial; ++i) BW_CHECK(o->initial_tokens[i] >= 0 && o->initial_tokens[i] < e->dims.n_vocab, "token id out of range");
+  if (lang) {
+    // upstream: is_multilingual = n_vocab >= 51865; an English-only model's sot sequence has no language token to detect
+    BW_CHECK(e->tt.num_languages > 0 && e->dims.n_vocab >= 51865,
+             "language detection: the model has no language tokens (English-only vocabulary)");
+    // upstream detect_language conditions on [sot] at position 0 alone: only then is the decode's sot row that row
+    BW_CHECK(o->sot_index == 0, "language detection: <|sot|> must be initial_tokens[0] (no prompt in front of it)");
+    BW_CHECK(o->n_initial >= 2 && o->initial_tokens[1] == kLanguagePlaceholder,
+             "language detection: initial_tokens[1] must be the language placeholder -1");
+  }
+  for (int i = 0; i < o->n_initial; ++i) {
+    if (lang && i == 1) continue;
+    BW_CHECK(!(lang && o->initial_tokens[i] == kLanguagePlaceholder),
+             "language detection: the placeholder -1 may only appear at initial_tokens[sot_index + 1]");
+    BW_CHECK(o->initial_tokens[i] >= 0 && o->initial_tokens[i] < e->dims.n_vocab, "token id out of range");
+  }
+  if (lang) {
+    memset(lang, 0, sizeof(*lang));
+    r.detect = true;
+    r.lang_out = lang;
+  }
   r.kind = REQ_DECODE;
   r.call = c;
   r.seek = seek;

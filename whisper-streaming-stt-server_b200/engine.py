@@ -48,10 +48,14 @@ def decode_opts(initial: Sequence[int], sot_index: int, beam_size: Optional[int]
     return o, init
 
 
-def result_dict(r: "L.ResultC") -> dict:
-    return {"tokens": list(r.tokens[: r.n_tokens]), "sum_logprob": r.sum_logprob, "avg_logprob": r.avg_logprob,
-            "no_speech_prob": r.no_speech_prob, "n_steps": r.n_steps, "t_queue": r.t_queue, "t_encode": r.t_encode,
-            "t_decode": r.t_decode}
+def result_dict(r: "L.ResultC", lang: Optional["L.LangResultC"] = None) -> dict:
+    d = {"tokens": list(r.tokens[: r.n_tokens]), "sum_logprob": r.sum_logprob, "avg_logprob": r.avg_logprob,
+         "no_speech_prob": r.no_speech_prob, "n_steps": r.n_steps, "t_queue": r.t_queue, "t_encode": r.t_encode,
+         "t_decode": r.t_decode}
+    if lang is not None:  # a detect-mode decode: the language it chose, as detect_language returns it
+        d["language_token"] = lang.language_token
+        d["language_probs"] = np.array(lang.probs[: lang.n_languages], dtype=np.float32)
+    return d
 
 
 class Call:
@@ -105,6 +109,20 @@ class Call:
         L.check(self.engine.lib.bw_call_detect_language(self._h, int(seek), C.byref(r)), "bw_call_detect_language")
         return r.language_token, np.array(r.probs[: r.n_languages], dtype=np.float32)
 
+    def decode_detect(self, seek: int, initial: Sequence[int], sot_index: int, beam_size: Optional[int], patience: Optional[float],
+                      length_penalty: Optional[float], sample_len: int = 0, without_timestamps: bool = False,
+                      suppress_blank: bool = True, max_initial_timestamp_index: Optional[int] = 50, temperature: float = 0.0,
+                      best_of: Optional[int] = None, seed: int = 0) -> dict:
+        """decode() of a window that detects its own language (bw_call_decode_detect): `initial` = [sot, LANGUAGE_PLACEHOLDER,
+        task, ...] with sot_index 0.  Returns decode()'s dict plus `language_token` and `language_probs` -- what
+        detect_language(seek) followed by decode() with that language's sot sequence return, for one encoder pass."""
+        o, _keep = decode_opts(initial, sot_index, beam_size, patience, length_penalty, sample_len, without_timestamps,
+                               suppress_blank, max_initial_timestamp_index, temperature, best_of, seed)
+        r, lang = L.ResultC(), L.LangResultC()
+        L.check(self.engine.lib.bw_call_decode_detect(self._h, int(seek), C.byref(o), C.byref(r), C.byref(lang)),
+                "bw_call_decode_detect")
+        return result_dict(r, lang)
+
     def close(self) -> None:
         if self._h:
             self.engine.lib.bw_call_close(self._h)
@@ -126,6 +144,9 @@ class Call:
 class Engine:
     """One weight copy + KV pools + scheduler thread on one GPU.  compute: "bf16" (product mode), "bf16_int8kv" (bf16 with the
     cached encoder K/V in 8 bits, BW_FLAG_CROSS_KV_INT8) or "fp32" (validation mode)."""
+
+    # Call.decode_detect / detect windows in decode_many: a window's decode can detect its own language
+    detects_in_decode = True
 
     def __init__(self, dims: ModelDims, state: Dict[str, object], device_index: int = 0, compute: str = "bf16",
                  max_segments: int = 0, max_sequences: int = 0, max_encoder_batch: int = 0, flags: int = 0, max_kv_pages: int = 0):
@@ -223,7 +244,8 @@ class Engine:
 
     def decode_many(self, items: Sequence[tuple]) -> list:
         """One blocking bw_decode_many for a batch of windows.  items[i] = (call, seek, kwargs of decode_opts); returns a
-        list of result dicts, or the B200WhisperError of the window that failed, in input order."""
+        list of result dicts, or the B200WhisperError of the window that failed, in input order.  A window whose kwargs
+        carry detect=True is a Call.decode_detect window (bw_decode_many_detect): its dict has the language too."""
         n = len(items)
         if n == 0:
             return []
@@ -231,13 +253,20 @@ class Engine:
         seeks = (C.c_int32 * n)(*[int(it[1]) for it in items])
         opts = (L.DecodeOptsC * n)()
         keep = []
+        detect = []
         for i, it in enumerate(items):
-            o, k = decode_opts(**it[2])
+            kw = dict(it[2])
+            detect.append(bool(kw.pop("detect", False)))
+            o, k = decode_opts(**kw)
             opts[i] = o
             keep.append(k)
         results = (L.ResultC * n)()
         statuses = (C.c_int32 * n)()
-        st = self.lib.bw_decode_many(calls, seeks, opts, results, statuses, n)
+        langs = (L.LangResultC * n)() if any(detect) else None
+        if langs is None:
+            st = self.lib.bw_decode_many(calls, seeks, opts, results, statuses, n)
+        else:
+            st = self.lib.bw_decode_many_detect(calls, seeks, opts, results, langs, statuses, n)
         if st != 0 and all(s == 0 for s in statuses):
             L.check(st, "bw_decode_many")
         out = []
@@ -247,7 +276,7 @@ class Engine:
                 out.append(L.B200WhisperError(f"bw_decode_many window {i} failed (bw_status {statuses[i]}): "
                                               f"{msg.decode('utf-8', 'replace') if msg else ''}"))
             else:
-                out.append(result_dict(results[i]))
+                out.append(result_dict(results[i], langs[i] if detect[i] else None))
         return out
 
     def stats(self) -> Dict[str, int]:
